@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — train samples/s (fwd+bwd) of the CTR hot path + unchanged torch tower on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--workload dcn] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload dcn] [--impl reference] [--dump-outputs DIR]
 
 One "step" = zero_grad, forward, loss, backward of the whole model on one synthetic
 WeChat-shaped batch (per-GPU batch fixed: weak scaling; for N > 1 the dense-gradient allreduce
@@ -18,6 +18,9 @@ is part of the step).  Rank 0 prints ONE JSON line (see DESIGN.md "Measurement")
               from a CUDA graph — the kernel-level bar of SURVEY.md §2.2 / §8d
   cpu_baseline / --impl reference : the oracle port of the reference model on the host cores
   other_workloads : one-line summaries of the other configurations (N = 1, default workload only)
+  --dump-outputs DIR : after the timed steps, what the last of them handed its caller (loss, forward
+              outputs, parameter gradients) as DIR/<name>.npy, so that two builds can be compared on the
+              same seeded inputs
 """
 from __future__ import annotations
 
@@ -40,6 +43,7 @@ import torch.nn.functional as F  # noqa: E402
 
 METRIC = "train samples/sec (fwd+bwd)"
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 64_000_000
 
 
 # ------------------------------------------------------------------------------- workloads
@@ -401,7 +405,41 @@ def dist_setup(n_gpus):
     return world, rank, local
 
 
-def cpu_reference_run(wl, steps, warmup, batch_size, budget_s=None):
+def capture_outputs(model):
+    """{"outputs": the tensors of the latest forward of `model`}.  Under a CUDA graph that is the captured
+    forward, whose outputs every replay rewrites in place.  Detached views: they keep no autograd graph alive."""
+    seen = {}
+
+    def hook(module, inputs, out):
+        seen["outputs"] = [o.detach() for o in ([out] if torch.is_tensor(out) else out) if torch.is_tensor(o)]
+
+    model.register_forward_hook(hook)
+    return seen
+
+
+def dump_outputs(out_dir, loss, outputs, model):
+    """What one training step hands its caller, one file per array: DIR/loss.npy, DIR/output_<i>.npy (the
+    forward's tensors) and DIR/grad.<parameter name>.npy, in float32 (float64 stays float64).  When they
+    exceed DUMP_BYTES in all, every array of more than one row keeps the same share of its rows, chosen by
+    a generator seeded with 0 and kept in ascending order, so two runs still compare row for row."""
+    import numpy as np
+    arrays = {"loss": loss}
+    arrays.update({f"output_{i}": o for i, o in enumerate(outputs)})
+    arrays.update({f"grad.{k}": p.grad for k, p in model.named_parameters() if p.grad is not None})
+    arrays = {k: v.detach().to(torch.float64 if v.dtype == torch.float64 else torch.float32).cpu().numpy()
+              for k, v in arrays.items()}
+    rows = {k for k, a in arrays.items() if a.ndim and a.shape[0] > 1}
+    whole = sum(a.nbytes for k, a in arrays.items() if k not in rows)
+    share = min(1.0, (DUMP_BYTES - whole) / max(sum(arrays[k].nbytes for k in rows), 1))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if share < 1.0 and name in rows:
+            keep = int(a.shape[0] * share)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def cpu_reference_run(wl, steps, warmup, batch_size, budget_s=None, dump_dir=None):
     """The oracle port of the reference model on the host cores: fwd + loss + bwd per step."""
     from oracle import models as oracle_models
     import rank_b200
@@ -411,6 +449,7 @@ def cpu_reference_run(wl, steps, warmup, batch_size, budget_s=None):
     torch.manual_seed(0)
     model = wl.model(oracle_models, True, vocab)
     model.train()
+    seen = capture_outputs(model) if dump_dir else None
     batches = [wl.make_batch(batch_size, 100 + i) for i in range(2)]
     times = []
     t_begin = time.perf_counter()
@@ -426,6 +465,8 @@ def cpu_reference_run(wl, steps, warmup, batch_size, budget_s=None):
             times.append(dt)
         if budget_s is not None and i >= warmup + 2 and time.perf_counter() - t_begin > budget_s:
             break
+    if seen is not None:
+        dump_outputs(dump_dir, loss, seen["outputs"], model)
     ms = 1e3 * sum(times) / len(times)
     return dict(value=batch_size / (ms / 1e3), ms_per_step=ms, steps=len(times), cores=threads,
                 loss=float(loss.detach()))
@@ -437,7 +478,7 @@ def run_reference(args, wl):
     if rank != 0:
         return
     B = args.batch or wl.batch
-    r = cpu_reference_run(wl, args.steps, args.warmup, B)
+    r = cpu_reference_run(wl, args.steps, args.warmup, B, dump_dir=args.dump_outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": r["value"], "unit": "samples/s",
         "n_gpus": args.gpus, "steps": r["steps"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"],
@@ -659,6 +700,7 @@ def measure_ours(args, wl, key, world, rank, local, dev, primary):
     torch.manual_seed(0)                    # identical replicas on every rank
     model = wl.model(rank_b200, False, vocab).to(dev)
     model.train()
+    seen = capture_outputs(model) if primary and args.dump_outputs else None
     reducer = GradientAllReducer(model) if world > 1 else None
 
     n_pool = 4
@@ -751,6 +793,8 @@ def measure_ours(args, wl, key, world, rank, local, dev, primary):
         host_value_ms = host_loop[0]
         barrier()
         clocks.mark()
+    if seen is not None and rank == 0:           # before the legs below reuse the step's buffers
+        dump_outputs(args.dump_outputs, stepper.loss, seen["outputs"], model)
     launches = stepper_launches_per_replay(stepper, lib) * steps if stepper.graph is not None else None
     # end to end: pinned host inputs -> H2D -> step -> D2H loss
     for i in range(3):
@@ -998,7 +1042,12 @@ def main():
     ap.add_argument("--no-others", action="store_true", help="skip the other workloads' one-line summaries")
     ap.add_argument("--calls", action="store_true", help="per-call event diagnostic for the other workloads too")
     ap.add_argument("--no-graph", action="store_true", help="launch every step eagerly instead of a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss, forward outputs and parameter "
+                         "gradients to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     claim_stdout()
     args.warmup = max(args.warmup, 3)
     wl = WORKLOADS[args.workload]()

@@ -43,6 +43,15 @@ def replay(model, fx, inputs, cotangents):
     return outs, grads
 
 
+def to_double(obj):
+    """The floating-point tensors of a fixture's inputs / cotangents in float64."""
+    if torch.is_tensor(obj):
+        return obj.double() if obj.is_floating_point() else obj
+    if isinstance(obj, dict):
+        return {k: to_double(v) for k, v in obj.items()}
+    return [to_double(v) for v in obj]
+
+
 def expand_sparse(entry):
     """A sparsely stored table of tests/golden/checkpoint_*.pt -> the full [height, dim] tensor
     (zeros in the rows the recorded batch never touches)."""

@@ -6,13 +6,22 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN_DIR, REFERENCE_ROOT, golden_files, grad_floor, load_golden, rel_err
+from conftest import GOLDEN_DIR, HAVE_REFERENCE, REFERENCE_ROOT, golden_files, grad_floor, load_golden, rel_err
 import golden_cases
 from oracle import interactions as X
 from oracle import models as oracle_models
 
 MODEL_FIXTURES = [p for p in golden_files() if "smoke" not in p and "loader" not in p and "checkpoint" not in p]
 TOL = 2e-6   # same torch ops in (almost) the same order: far inside the 1e-5 bar
+BAR = 1e-5   # the project's fp32 parity bar
+ZERO = 1e-4  # a gradient below ZERO x the model's largest one is mathematically zero: rounding noise only
+
+
+def _oracle_grads_float64(fx, vocab_dir):
+    model = golden_cases.build(fx, oracle_models, vocab_dir, oracle=True)
+    model.load_state_dict(fx["state_dict"], strict=True)
+    return golden_cases.replay(model.double(), fx, golden_cases.to_double(fx["inputs"]),
+                               golden_cases.to_double(fx["cotangents"]))[1]
 
 
 @pytest.mark.parametrize("path", MODEL_FIXTURES, ids=[os.path.basename(p) for p in MODEL_FIXTURES])
@@ -30,8 +39,29 @@ def test_oracle_matches_reference_fixture(path, small_vocab_dir):
             assert o == ref
     assert set(grads) == set(fx["grads"])
     floor = grad_floor(fx["grads"])
+    gmax = max(float(g.abs().max()) for g in fx["grads"].values())
+    grads64 = None
     for k, g in fx["grads"].items():
-        assert rel_err(grads[k], g, floor) <= TOL, k
+        e = rel_err(grads[k], g, floor)
+        if e <= TOL:
+            continue
+        # The recorded gradients carry the summation order of the host that recorded them; with another
+        # thread count or vector width the CPU kernels add the same terms in another order.
+        if float(g.abs().max()) < ZERO * gmax:
+            # mathematically zero (a Linear bias feeding BatchNorm): both sides hold only the rounding noise
+            # of cancelling sums, so the bar is taken against the model's gradient scale, as in
+            # tests/test_gpu_models.py::compare
+            err = float((grads[k].double() - g.double()).abs().max())
+            assert err <= TOL * gmax, f"grad {k} (numerically zero): abs err {err / gmax:.3e} of the scale"
+        else:
+            # both fp32 results against the oracle in float64: the recorded one must lie within the 1e-5 bar
+            # of it (the oracle does the reference's arithmetic) and the oracle's own fp32 result no further
+            # from it than TOL or twice the recorded one's rounding error
+            if grads64 is None:
+                grads64 = _oracle_grads_float64(fx, small_vocab_dir)
+            e_ref, e_ours = rel_err(g, grads64[k], floor), rel_err(grads[k], grads64[k], floor)
+            assert e_ref <= BAR and e_ours <= max(TOL, 2.0 * e_ref), \
+                f"grad {k}: {e:.3e} vs recorded; vs float64: oracle {e_ours:.3e}, recorded {e_ref:.3e}"
 
 
 def test_din_attention_reference_smoke():
@@ -64,7 +94,8 @@ def test_stable_occurrence_order():
     assert perm.tolist() == [1, 3, 0, 2, 0, 1]
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_ROOT), reason="reference checkout not present")
+@pytest.mark.skipif(not HAVE_REFERENCE, reason="needs the reference checkout (RANK_REFERENCE_ROOT); "
+                    "test_oracle_matches_shipped_checkpoint_fixture checks the same checkpoints against its recorded outputs")
 @pytest.mark.parametrize("which", ["DCN", "DeepCrossing"])
 def test_oracle_loads_shipped_checkpoint_and_matches_reference(which):
     """The two real trained state_dicts the reference ships, on the real vocabulary sizes."""

@@ -206,7 +206,7 @@ def _nccl_worker(rank, world, port, vocab_dir, out):
 def test_sharded_bst_two_ranks_nccl(wechat_vocab_dir):
     """The all-to-all path proper (needs two GPUs; the one-GPU box runs the world-1 tests above)."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     ctx = mp.get_context("spawn")
     out = ctx.SimpleQueue()
     port = _free_port()
@@ -262,7 +262,7 @@ def _exchange_worker(rank, world, port, vocab_dir, out):
 @pytest.mark.gpu
 def test_occurrence_exchange_matches_dense_allreduce_two_ranks(wechat_vocab_dir):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     ctx = mp.get_context("spawn")
     out = ctx.SimpleQueue()
     port = _free_port()
