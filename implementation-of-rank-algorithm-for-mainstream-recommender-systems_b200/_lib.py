@@ -19,7 +19,7 @@ RK_MAX_FIELDS = 24
 RK_MAX_TABLES = 32
 RK_MAX_LAYERS = 8
 RK_DIRECT_MAX_N = 8192
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class RkField(C.Structure):
@@ -102,7 +102,6 @@ PROTOTYPES = {
     "rk_rowwise_adam": (_I, [_P, _P, _P, _P, _P, _L, _I, _L, _F, _F, _F, _F, _L, _P, _P]),
     "rk_shard_owner": (_I, [_P, _L, _L, _L, _P, _P, _P]),
     "rk_shard_route": (_I, [_P, _P, _P, _L, _L, _L, _I, _P, _P, _P, _P]),
-    "rk_plan_compact": (_I, [_P, _L, _L, _P, _P, _P, _P]),
     "rk_plan_compact_fields": (_I, [_P, _P, _P, _P, _I, _P, _P, _P, _P]),
     "rk_rowwise_adam_touched": (_I, [_P, _P, _P, _P, _P, _P, _L, _I, _L, _F, _F, _F, _F, _L, _P, _P]),
     "rk_resunit_pack_floats": (_I, [_I, _I]),

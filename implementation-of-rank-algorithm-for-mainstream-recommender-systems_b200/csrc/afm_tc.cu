@@ -8,7 +8,6 @@
 // Operand tiles: one 128-byte line per row holding [hi(Kp) | lo(Kp)] bf16 (Kp = D rounded up to
 // 16, <= 32), so the three split terms are three (A k-slice, B k-slice) pairings of the same two
 // tiles.  HBM traffic is the same as the SIMT kernel's (idx + rows in, out written once).
-#include <stdlib.h>
 #include <string.h>
 #include "common.cuh"
 #include "umma.cuh"
@@ -30,7 +29,7 @@ struct AfmTcParams {
     const float* b2;   // [1]
     int32_t      D, Kp, A, Ap, P, S, estride;
     int64_t      B, n_tiles;
-    const uint8_t* tiles;   // prologue-made operand tiles (afm_weight_tiles_kernel) or NULL: convert per CTA
+    const uint8_t* tiles;   // operand tiles made once per forward by afm_weight_tiles_kernel
 };
 
 // Image written once per forward by afm_weight_tiles_kernel and fetched by one / two bulk (TMA) copies per CTA:
@@ -121,7 +120,7 @@ __device__ __forceinline__ void afm_issue_rows(const AfmTcParams& p, float* e, c
     }
 }
 
-// ---- the weight operand tiles (shared memory in the per-CTA path, the global image in the prologue kernel)
+// ---- the weight operand tiles, written into the global image by afm_weight_tiles_kernel
 // B1 line n = [hi | lo] of W1[n][:], zero beyond A / D
 template <int KP>
 __device__ __forceinline__ void afm_build_b1(uint8_t* b1t, const float* __restrict__ w1, int A, int D, int lines, int tid,
@@ -213,13 +212,10 @@ afm_fwd_tc_kernel(const __grid_constant__ AfmTcParams p, float* __restrict__ out
     if (tid == 0) {
         mbar_init(sm.bar, 1);
         mbar_init(sm.bar_w, 1);
-        if (p.tiles) {                     // W1's operand tile in one bulk (TMA) copy
-            mbar_expect_tx(sm.bar_w, (uint32_t)p.Ap * 128u);
-            bulk_copy_g2s(sm.b1t, p.tiles, (uint32_t)p.Ap * 128u, sm.bar_w);
-        }
+        mbar_expect_tx(sm.bar_w, (uint32_t)p.Ap * 128u);          // W1's operand tile in one bulk (TMA) copy
+        bulk_copy_g2s(sm.b1t, p.tiles, (uint32_t)p.Ap * 128u, sm.bar_w);
     }
     if (warp == 0) tmem_alloc(sm.tmem_slot, 128);
-    if (!p.tiles) afm_build_b1<KP>(sm.b1t, p.w1, p.A, D, p.Ap, tid, kAfmTcThreads);
     for (int n = tid; n < p.Ap; n += kAfmTcThreads) {
         sm.bias[n] = n < p.A ? __ldg(p.b1 + n) : 0.f;
         sm.w2[n]   = n < p.A ? __ldg(p.w2 + n) : 0.f;
@@ -233,7 +229,7 @@ afm_fwd_tc_kernel(const __grid_constant__ AfmTcParams p, float* __restrict__ out
     fence_before();
     __syncthreads();
     fence_after();
-    if (p.tiles) mbar_wait(sm.bar_w, 0);
+    mbar_wait(sm.bar_w, 0);
     const uint32_t tmem = *sm.tmem_slot;
     const uint32_t my_tmem = tmem + ((uint32_t)(warp * 32) << 16);
     const uint64_t a_desc = umma_desc(smem_u32(sm.a1)), b_desc = umma_desc(smem_u32(sm.b1t));
@@ -479,35 +475,16 @@ afm_bwd_tc_kernel(const __grid_constant__ AfmTcParams p, const float* __restrict
     if (tid == 0) {
         mbar_init(sm.bar, 1);
         mbar_init(sm.bar_w, 1);
-        if (p.tiles) {                     // B1 and B2 in two bulk (TMA) copies on one barrier
-            mbar_expect_tx(sm.bar_w, kAfmTileB1 + kAfmTileB2);
-            bulk_copy_g2s(sm.b1t, p.tiles, kAfmTileB1, sm.bar_w);
-            bulk_copy_g2s(sm.b2t, p.tiles + kAfmTileB1, kAfmTileB2, sm.bar_w);
-            sm.wmax[0] = __ldg(reinterpret_cast<const float*>(p.tiles + kAfmTileB1 + kAfmTileB2));
-        }
+        mbar_expect_tx(sm.bar_w, kAfmTileB1 + kAfmTileB2);        // B1 and B2 in two bulk (TMA) copies on one barrier
+        bulk_copy_g2s(sm.b1t, p.tiles, kAfmTileB1, sm.bar_w);
+        bulk_copy_g2s(sm.b2t, p.tiles + kAfmTileB1, kAfmTileB2, sm.bar_w);
+        // max |W1|: scales the band around zero inside which a pre-activation is recomputed in fp32
+        sm.wmax[0] = __ldg(reinterpret_cast<const float*>(p.tiles + kAfmTileB1 + kAfmTileB2));
     }
     if (warp == 0) tmem_alloc(sm.tmem_slot, 256);
     for (int n = tid; n < 128; n += kAfmTcThreads) {
         sm.bias[n] = n < A ? __ldg(p.b1 + n) : 0.f;
         sm.w2[n]   = n < A ? __ldg(p.w2 + n) : 0.f;
-    }
-    if (!p.tiles) {                        // per-CTA conversion (no prologue image)
-        afm_build_b1<KP>(sm.b1t, p.w1, A, D, 128, tid, kAfmTcThreads);
-        for (int i = tid; i < 2 * 64 * 128 / 16; i += kAfmTcThreads)
-            reinterpret_cast<uint4*>(sm.b2t)[i] = make_uint4(0u, 0u, 0u, 0u);
-        __syncthreads();
-        afm_scatter_b2<KP>(sm.b2t, p.w1, p.w2, A, D, tid, kAfmTcThreads);
-        // max |W1|: scales the band around zero inside which a pre-activation is recomputed in fp32
-        float m = 0.f;
-        for (int i = tid; i < A * D; i += kAfmTcThreads) m = fmaxf(m, fabsf(__ldg(p.w1 + i)));
-        m = warp_max(m);
-        if (lane == 0) sm.red[warp] = m;
-        __syncthreads();
-        if (tid == 0) {
-            float t = 0.f;
-            for (int w = 0; w < kAfmTcThreads / 32; ++w) t = fmaxf(t, sm.red[w]);
-            sm.wmax[0] = t;
-        }
     }
     for (int i = tid; i < 2 * 128 * 128 / 16; i += kAfmTcThreads)       // mask columns >= Ap stay zero
         reinterpret_cast<uint4*>(sm.a2)[i] = make_uint4(0u, 0u, 0u, 0u);
@@ -528,7 +505,7 @@ afm_bwd_tc_kernel(const __grid_constant__ AfmTcParams p, const float* __restrict
     fence_before();
     __syncthreads();
     fence_after();
-    if (p.tiles) mbar_wait(sm.bar_w, 0);
+    mbar_wait(sm.bar_w, 0);
     const uint32_t tmem = *sm.tmem_slot;
     const uint32_t my_tmem = tmem + ((uint32_t)(warp * 32) << 16);
     const uint64_t a1_desc = umma_desc(smem_u32(sm.a1)), b1_desc = umma_desc(smem_u32(sm.b1t));
@@ -874,6 +851,7 @@ afm_bwd_tc_kernel(const __grid_constant__ AfmTcParams p, const float* __restrict
 
 static int afm_tc_fill(const rk_field_t* fields, int F, const float* w1, const float* b1, const float* w2,
                        const float* b2, int A, int64_t B, const void* tiles, tc::AfmTcParams* p) {
+    RK_CHECK_ARG(tiles, "afm: tiles is NULL (rk_afm_tile_bytes() bytes of scratch are required)");
     RK_CHECK_ARG(((uintptr_t)tiles % 128) == 0, "afm: tiles must be 128-byte aligned");
     p->tiles = (const uint8_t*)tiles;
     if (int rc = pack_fields(fields, F, &p->fs)) return rc;
@@ -916,19 +894,14 @@ int rk_afm_tc_fwd(const rk_field_t* fields, int F, const float* w1, const float*
     // (a second wave would redo the per-CTA set-up).  cudaOccupancyMaxActiveBlocksPerMultiprocessor
     // reports 1 for kernels that allocate TMEM, so the bound is stated here: 4 x 128 TMEM columns,
     // 4 x 128 threads x 128 registers, 4 x ~44 KB of shared memory per SM.
-    static const int occ = [] {
-        const char* e = getenv("RANK_B200_AFM_TC_CTAS_PER_SM");
-        const int v = e ? atoi(e) : 0;
-        return v >= 1 && v <= 4 ? v : 4;
-    }();
+    constexpr int occ = 4;
     int64_t grid = p.n_tiles;
     const int64_t cap = (int64_t)sm_count() * occ;
     if (grid > cap) grid = cap;
-    if (tiles) {                           // both directions' weight tiles, once per forward
-        if (p.Kp == 16) tc::afm_weight_tiles_kernel<16><<<2, 256, 0, (cudaStream_t)stream_>>>(w1, w2, A, p.D, (uint8_t*)tiles);
-        else            tc::afm_weight_tiles_kernel<32><<<2, 256, 0, (cudaStream_t)stream_>>>(w1, w2, A, p.D, (uint8_t*)tiles);
-        RK_LAUNCH_CHECK();
-    }
+    // both directions' weight tiles, once per forward
+    if (p.Kp == 16) tc::afm_weight_tiles_kernel<16><<<2, 256, 0, (cudaStream_t)stream_>>>(w1, w2, A, p.D, (uint8_t*)tiles);
+    else            tc::afm_weight_tiles_kernel<32><<<2, 256, 0, (cudaStream_t)stream_>>>(w1, w2, A, p.D, (uint8_t*)tiles);
+    RK_LAUNCH_CHECK();
     kernel<<<(int)grid, tc::kAfmTcThreads, smem, (cudaStream_t)stream_>>>(p, out, err_flag);
     RK_LAUNCH_CHECK();
     return 0;

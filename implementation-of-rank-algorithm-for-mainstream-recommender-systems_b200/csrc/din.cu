@@ -37,7 +37,7 @@ struct DinParams {
     const int64_t* his_len;
     int32_t        T, D, att_off, width, l2_from, use_softmax;
     const float*   mlp;
-    const uint8_t* mlp_tiles;               // prologue-made operand tiles (tensor-core path), or NULL
+    const uint8_t* mlp_tiles;               // operand tiles made once per forward (tensor-core path)
     int64_t        B;
 };
 
@@ -749,26 +749,11 @@ din_fwd_tc_kernel(const __grid_constant__ DinParams p, float* __restrict__ conca
     if (tid == 0) {
         mbar_init(sm.bar_mma, 1);
         mbar_init(sm.bar_w, 1);
-        if (p.mlp_tiles) {            // the four weight tiles in one bulk (TMA) copy: w1 | w1_lo | w2 | w2_lo are contiguous
-            mbar_expect_tx(sm.bar_w, kTileFwdBytes);
-            bulk_copy_g2s(sm.w1, p.mlp_tiles, kTileFwdBytes, sm.bar_w);
-        }
+        // the four weight tiles in one bulk (TMA) copy: w1 | w1_lo | w2 | w2_lo are contiguous
+        mbar_expect_tx(sm.bar_w, kTileFwdBytes);
+        bulk_copy_g2s(sm.w1, p.mlp_tiles, kTileFwdBytes, sm.bar_w);
     }
     if (warp == 0) tmem_alloc(sm.tmem_slot, kTcTmemCols);
-    if (!p.mlp_tiles) {
-        for (int item = tid; item < 64 * 8; item += kTcThreads) {         // W1[n][k]: 64 rows x 8 chunks
-            const int n = item >> 3, c = item & 7;
-            float v[8];
-            ld8(p.mlp + L.w1 + n * 64 + c * 8, v);
-            store_chunk_split(sm.w1, sm.w1_lo, n, c, v);
-        }
-        for (int item = tid; item < 32 * 8; item += kTcThreads) {         // W2[n][k]: 32 rows x 8 chunks
-            const int n = item >> 3, c = item & 7;
-            float v[8];
-            ld8(p.mlp + L.w2 + n * 64 + c * 8, v);
-            store_chunk_split(sm.w2, sm.w2_lo, n, c, v);
-        }
-    }
     for (int i = tid; i < kH1; i += kTcThreads) sm.vec[i] = __ldg(p.mlp + L.b1 + i);
     for (int i = tid; i < kH2; i += kTcThreads) {
         sm.vec[kH1 + i]       = __ldg(p.mlp + L.b2 + i);
@@ -786,7 +771,7 @@ din_fwd_tc_kernel(const __grid_constant__ DinParams p, float* __restrict__ conca
     fence_before();
     __syncthreads();
     fence_after();
-    if (p.mlp_tiles) mbar_wait(sm.bar_w, 0);
+    mbar_wait(sm.bar_w, 0);
     const uint32_t tmem = *sm.tmem_slot;
     const float* b1 = sm.vec;
     const float* b2 = sm.vec + kH1;
@@ -1222,32 +1207,17 @@ din_bwd_tc_kernel(const __grid_constant__ DinParams p, const float* __restrict__
     if (tid == 0) {
         mbar_init(sm.bar, 1);
         mbar_init(sm.bar_w, 1);
-        if (p.mlp_tiles) {            // w1 | w1_lo | w2 | w2_lo (W1^T, W2^T) in one bulk (TMA) copy
-            mbar_expect_tx(sm.bar_w, kTileBwdBytes);
-            bulk_copy_g2s(sm.w1, p.mlp_tiles + kTileFwdBytes, kTileBwdBytes, sm.bar_w);
-        }
+        // w1 | w1_lo | w2 | w2_lo (W1^T, W2^T) in one bulk (TMA) copy
+        mbar_expect_tx(sm.bar_w, kTileBwdBytes);
+        bulk_copy_g2s(sm.w1, p.mlp_tiles + kTileFwdBytes, kTileBwdBytes, sm.bar_w);
     }
     if (warp == 0) tmem_alloc(sm.tmem_slot, kTcTmemCols);
-    if (!p.mlp_tiles) {
-        for (int item = tid; item < 64 * 4; item += kTcThreads) {          // W2^T[n][k]: 64 rows x 32 k (4 chunks)
-            const int n = item >> 2, c = item & 3;
-            float v[8];
-            ld8(p.mlp + L.w2t + n * 32 + c * 8, v);
-            store_chunk_split(sm.w2, sm.w2_lo, n, c, v);
-        }
-        for (int item = tid; item < 64 * 8; item += kTcThreads) {          // W1^T[c][n]: 64 rows x 64 k
-            const int n = item >> 3, c = item & 7;
-            float v[8];
-            ld8(p.mlp + L.w1t + n * 64 + c * 8, v);
-            store_chunk_split(sm.w1, sm.w1_lo, n, c, v);
-        }
-    }
     for (int i = tid; i < kH2; i += kTcThreads) sm.vec[i] = __ldg(p.mlp + L.w3 + i);
     fence_async_smem();
     fence_before();
     __syncthreads();
     fence_after();
-    if (p.mlp_tiles) mbar_wait(sm.bar_w, 0);
+    mbar_wait(sm.bar_w, 0);
     const uint32_t tmem = *sm.tmem_slot;
     const float* w3 = sm.vec;
     const uint64_t a_desc[2]  = {umma_desc(smem_u32(sm.a)), umma_desc(smem_u32(sm.a_lo))};
@@ -1510,6 +1480,8 @@ static int din_pack(const rk_din_args_t* a, rk::DinParams* p) {
     p->l2_from = a->l2_from;  p->use_softmax = a->use_softmax;
     p->mlp = a->mlp;  p->B = a->B;
     p->mlp_tiles = (const uint8_t*)a->mlp_tiles;
+    RK_CHECK_ARG(a->precision != RK_DIN_BF16_TENSOR || a->mlp_tiles,
+                 "din: mlp_tiles is NULL (RK_DIN_BF16_TENSOR needs rk_din_tile_bytes() bytes of scratch)");
     RK_CHECK_ARG(((uintptr_t)a->mlp_tiles % 128) == 0, "din: mlp_tiles must be 128-byte aligned");
     RK_CHECK_ARG(p->width > 0 && p->att_off + D <= p->width && p->tgt_off + D <= p->width, "din: bad layout");
     return 0;
@@ -1534,11 +1506,7 @@ int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float*
     if (args->precision == RK_DIN_BF16_TENSOR) {
         RK_CHECK_ARG(p.D == 16, "din_fwd: the tensor-core activation unit is built for D = 16 (got %d)", p.D);
         const size_t smem_tc = tc::TcFwdSmem::bytes(p.width, p.T, p.cat.F);
-        static const int per_sm = [] {
-            const char* e = getenv("RANK_B200_DIN_TC_CTAS_PER_SM");
-            const int v = e ? atoi(e) : 0;
-            return v >= 1 && v <= 4 ? v : 3;
-        }();
+        constexpr int per_sm = 3;
         auto kernel = tc::din_fwd_tc_kernel;
         RK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tc));
         // Persistent CTAs drawing groups of samples from a device-side counter: static striding was
@@ -1546,10 +1514,9 @@ int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float*
         // history lengths; dynamic draws keep the balance and pay the per-CTA setup once.
         const int n_groups = (int)ceil_div(p.B, tc::kTcGroup);
         const int grid_tc = n_groups < sm_count() * per_sm ? n_groups : sm_count() * per_sm;
-        if (p.mlp_tiles) {            // both directions' operand tiles, once per forward
-            tc::din_weight_tiles_kernel<<<6, 256, 0, (cudaStream_t)stream_>>>(p.mlp, (uint8_t*)args->mlp_tiles);
-            RK_LAUNCH_CHECK();
-        }
+        // both directions' operand tiles, once per forward
+        tc::din_weight_tiles_kernel<<<6, 256, 0, (cudaStream_t)stream_>>>(p.mlp, (uint8_t*)args->mlp_tiles);
+        RK_LAUNCH_CHECK();
         kernel<<<grid_tc, tc::kTcThreads, smem_tc, (cudaStream_t)stream_>>>(
             p, concat_all, norm, att_w, relu_masks, err_flag);
         RK_LAUNCH_CHECK();
@@ -1588,11 +1555,7 @@ int rk_din_bwd(const rk_din_args_t* args, const float* concat_all, const float* 
         RK_CUDA(cudaFuncSetAttribute(tc::din_bwd_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                      (int)cudaSharedmemCarveoutMaxShared));
         // persistent CTAs, two per SM by shared memory; the grid never exceeds the group count
-        static const int per_sm = [] {
-            const char* e = getenv("RANK_B200_DIN_TC_BWD_CTAS_PER_SM");
-            const int v = e ? atoi(e) : 0;
-            return v >= 1 && v <= 4 ? v : 2;
-        }();
+        constexpr int per_sm = 2;
         const int grid_tc = grid < sm_count() * per_sm ? grid : sm_count() * per_sm;
         tc::din_bwd_tc_kernel<<<grid_tc, tc::kTcThreads, smem_tc, (cudaStream_t)stream_>>>(
             p, concat_all, norm, att_w, relu_masks, g_concat, g_norm, g_row, g_hist, err_flag);

@@ -6,9 +6,6 @@
 //   rk_shard_route   : from the stable owner-sorted order (rk_plan_build on owner[]) produce the
 //                      send buffer of owner-local row ids, the inverse permutation and the
 //                      per-owner counts
-//   rk_plan_compact  : dense ranks of the sorted keys + the list of unique rows, so that the
-//                      segment reduction can write a compact [unique, D] gradient (sparse update
-//                      of a shard far too large for a dense gradient)
 // Integer, latency-bound work on a few hundred thousand elements per step.
 #include "common.cuh"
 
@@ -132,24 +129,6 @@ int rk_shard_route(const int64_t* idx, const uint32_t* sorted_owner, const uint3
     if (grid > (int64_t)sm_count() * 4) grid = (int64_t)sm_count() * 4;
     shard_route_kernel<<<(int)grid, 256, 0, s>>>(idx, sorted_owner, perm, n, rows_total, rows_per_rank, W,
                                                  send_local, inv, counts);
-    RK_LAUNCH_CHECK();
-    return 0;
-}
-
-int rk_plan_compact(const uint32_t* sorted_keys, int64_t n, int64_t rows, uint32_t* rank_keys, int64_t* uniq_rows,
-                    int64_t* n_uniq, rk_stream_t stream_) {
-    using namespace rk;
-    RK_CHECK_ARG(n >= 0 && rows > 0 && n_uniq, "plan_compact: bad argument");
-    cudaStream_t s = (cudaStream_t)stream_;
-    if (n == 0) {
-        RK_CUDA(cudaMemsetAsync(n_uniq, 0, sizeof(int64_t), s));
-        return 0;
-    }
-    RK_CHECK_ARG(sorted_keys && rank_keys && uniq_rows, "plan_compact: NULL pointer");
-    // single-field plan: key_base = 0, dead key = rows; dead positions get the sentinel rank 0xffffffff
-    CompactFields cf;
-    cf.f[0] = CompactField{0, n, 0u, (uint32_t)rows, 0u, 0xffffffffu};
-    plan_compact_kernel<<<1, 1024, 0, s>>>(sorted_keys, cf, rank_keys, uniq_rows, n_uniq);
     RK_LAUNCH_CHECK();
     return 0;
 }

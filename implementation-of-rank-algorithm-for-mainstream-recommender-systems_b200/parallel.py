@@ -10,9 +10,6 @@ back as views of that buffer (no copy back).
 """
 from __future__ import annotations
 
-import os
-import warnings
-
 import torch
 import torch.distributed as dist
 
@@ -27,14 +24,11 @@ class GradientAllReducer:
     itself (ReduceOp.AVG; gloo: SUM then one scale).  Every call is stream-ordered device work — the whole
     step including the collective can be captured in a CUDA graph (bench.py does)."""
 
-    def __init__(self, model: torch.nn.Module, group=None, attach=True, occurrence_exchange=None):
+    # bench.py reports it; the collective is always torch.distributed's (NCCL, or gloo in the CPU tests)
+    symmetric = None
+
+    def __init__(self, model: torch.nn.Module, group=None, attach=True):
         self.group = group
-        # opt-in (or RANK_B200_OCCURRENCE_EXCHANGE=1): see _exchange_occurrences.  Measured at 2 GPUs on DeepFM
-        # (batch 1024 per rank): 13.5 MB all-reduced -> 0.9 MB all-gathered, and the step stays at 0.339 ms either
-        # way - at this size the cost of a collective is its fixed latency and the skew between the ranks'
-        # independently launched graphs, not its bytes - so the dense all-reduce remains the default.
-        self.occurrence_exchange = (os.environ.get("RANK_B200_OCCURRENCE_EXCHANGE", "0") == "1"
-                                    if occurrence_exchange is None else bool(occurrence_exchange))
         # row-sharded tables are owned by one rank each: their gradients are not replicated
         self.params = [p for p in model.parameters()
                        if p.requires_grad and not getattr(p, "_rank_local", False)]
@@ -45,15 +39,7 @@ class GradientAllReducer:
         self.n_staging = (sum(sizes) + 31) // 32 * 32          # the table region starts 128-byte aligned
         # table region: every parameter could be a table, each slab padded to 16 bytes per table
         self.n_slab = sum(sizes) + 4 * len(sizes)
-        total = (self.n_staging + self.n_slab + 1023) // 1024 * 1024 + 1024      # room to round the reduced range
-        # RANK_B200_ALLREDUCE = nccl (default) | two_shot | multimem: the collective can also run as one of torch's
-        # symmetric-memory kernels over peer-mapped memory (two-shot reduce-scatter + all-gather through P2P loads,
-        # or NVSwitch multicast); the buffer is then symmetric memory.  Measured on this box for DIN's 16.7 MB at 2
-        # GPUs (profiles/r02_scaling.md): NCCL 0.949 ms per step, two_shot 0.961, multimem 1.04 - NCCL stays the default.
-        self.symmetric = None
-        self.flat = self._symmetric_buffer(total, dtype, dev)
-        if self.flat is None:
-            self.flat = torch.zeros(total, dtype=dtype, device=dev)
+        self.flat = torch.zeros(self.n_staging + self.n_slab, dtype=dtype, device=dev)
         self.views, pos = [], 0
         for p, n in zip(self.params, sizes):
             self.views.append(self.flat[pos:pos + n].view_as(p))
@@ -68,147 +54,14 @@ class GradientAllReducer:
     def world_size(self):
         return dist.get_world_size(self.group)
 
-    # ---- symmetric-memory all-reduce (torch.distributed._symmetric_memory: library kernels over NVLink peers)
-    def _symmetric_buffer(self, total, dtype, dev):
-        mode = os.environ.get("RANK_B200_ALLREDUCE", "nccl")
-        if mode not in ("two_shot", "multimem") or dev.type != "cuda" or not dist.is_initialized() or dist.get_backend(self.group) != "nccl" \
-                or dist.get_world_size(self.group) < 2:
-            return None
-        buf = None
-        kinds = []
-        try:
-            import torch.distributed._symmetric_memory as symm
-            group = self.group if self.group is not None else dist.group.WORLD
-            name = group.group_name
-            buf = symm.empty(total, dtype=dtype, device=dev)
-            handle = symm.rendezvous(buf, group)
-            buf.zero_()
-            has_multicast = bool(getattr(handle, "multicast_ptr", 0))
-            kinds = [k for k in [mode] if k != "multimem" or has_multicast]
-        except Exception as exc:          # no symmetric memory on this build / fabric: NCCL it is
-            warnings.warn(f"rank_b200: symmetric-memory all-reduce unavailable ({type(exc).__name__}: {exc}); using NCCL")
-            buf, kinds = None, []
-        # every rank must take the same path: agree on the first kind that reproduces NCCL's result everywhere
-        chosen = None
-        for kind in ["multimem", "two_shot"]:
-            ok = 0.0
-            if buf is not None and kind in kinds:
-                try:
-                    ok = float(self._symmetric_selftest(buf, kind, name))
-                except Exception as exc:
-                    warnings.warn(f"rank_b200: {kind} all-reduce failed its self-test ({type(exc).__name__}: {exc})")
-            flag = torch.tensor([ok], device=dev)
-            dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
-            if float(flag) > 0.5:
-                chosen = kind
-                break
-        if chosen is None:
-            return None
-        self.symmetric = (chosen, name)
-        buf.zero_()
-        return buf
-
-    def _symmetric_selftest(self, buf, kind, name):
-        n = min(int(buf.numel()), 1 << 20) // 1024 * 1024
-        rank, world = dist.get_rank(self.group), dist.get_world_size(self.group)
-        base = torch.arange(n, device=buf.device, dtype=torch.float32) % 1000 / 1000.0
-        view = buf[:n]
-        view.copy_(base * (rank + 1))
-        torch.cuda.synchronize()
-        self._symmetric_allreduce(view, kind, name)
-        torch.cuda.synchronize()
-        want = base * (world * (world + 1) / 2)
-        return bool(torch.allclose(view, want, rtol=1e-5, atol=1e-6))
-
-    @staticmethod
-    def _symmetric_allreduce(view, kind, name):
-        if kind == "multimem":
-            torch.ops.symm_mem.multimem_all_reduce_(view, "sum", name)
-        else:
-            torch.ops.symm_mem.two_shot_all_reduce_(view, "sum", name)
-
-    def use_nccl(self):
-        """Fall back to the NCCL collective (e.g. when a CUDA-graph capture of the symmetric-memory kernels fails)."""
-        self.symmetric = None
-
     # ---- slab provider of rank_b200.sparse ------------------------------------------------------
     def attach(self):
         from . import sparse
         sparse.set_slab_provider(self._take)
-        sparse.set_occurrence_exchange(self._exchange_occurrences if self.occurrence_exchange else None)
 
     def detach(self):
         from . import sparse
         sparse.set_slab_provider(None)
-        sparse.set_occurrence_exchange(None)
-
-    # ---- small batches: exchange the occurrences, not the tables -----------------------------------
-    def _exchange_occurrences(self, plan, sources):
-        """DeepFM / FwFM at their BASELINE batch of 1024: a rank touches <= 6 144 of 213 k table rows per step, yet
-        the dense gradients are 13 MB.  When world x n occurrences fit one direct reduction (<= 8192 per index
-        column) the ranks all-gather (index, gradient row / world) — ~0.45 MB per rank — and every rank reduces
-        the occurrences of the whole global batch, rank-major, in occurrence order: the result is the averaged
-        gradient, bit-identical on all ranks, and those tables never enter the all-reduce."""
-        from . import _lib, sparse
-        if not dist.is_initialized():
-            return None
-        world = self.world_size
-        if world < 2 or not sources or plan.device != self.flat.device:
-            return None
-        n = plan.n[sources[0].field]
-        if n == 0 or world * n > _lib.RK_DIRECT_MAX_N:
-            return None
-        for s in sources:
-            if (not plan.direct[s.field] or plan.n[s.field] != n or s.param is None
-                    or id(s.param) not in self._param_ids or s.base.dtype != torch.float32):
-                return None
-        dev = plan.device
-        fields = sorted({s.field for s in sources})
-        fpos = {f: k for k, f in enumerate(fields)}
-        F = len(fields)
-        # columns of the packed gradient rows: sources that read the same columns share them (DeepFM's six
-        # first-order tables all receive the same per-sample scalar), adjacent columns of one tensor are one copy
-        cols, spans, seen, width = [], [], {}, 0
-        for s in sources:
-            key = (s.base.data_ptr(), s.offset, s.dim, s.ld)
-            if key in seen:
-                cols.append(seen[key])
-                continue
-            seen[key] = width
-            cols.append(width)
-            last = spans[-1] if spans else None
-            if last is not None and last[0] is s.base and last[3] == s.ld and last[1] + last[2] == s.offset:
-                last[2] += s.dim
-            else:
-                spans.append([s.base, s.offset, s.dim, s.ld, width])
-            width += s.dim
-        # one packed message per rank: [F, n] int64 indices | [n, width] fp32 gradient rows scaled by 1 / world
-        idx_bytes, g_bytes = F * n * 8, n * width * 4
-        send = torch.empty(idx_bytes + g_bytes, dtype=torch.uint8, device=dev)
-        send_idx = send[:idx_bytes].view(torch.int64).view(F, n)
-        send_g = send[idx_bytes:].view(torch.float32).view(n, width)
-        torch.stack([plan.indices[f].reshape(-1) for f in fields], out=send_idx)
-        for base, off, dim, ld, pos in spans:
-            rows_view = torch.as_strided(base, (n, dim), (ld, 1), base.storage_offset() + off)
-            send_g[:, pos:pos + dim].copy_(rows_view)
-        send_g.mul_(1.0 / world)
-        recv = torch.empty(world, idx_bytes + g_bytes, dtype=torch.uint8, device=dev)
-        dist.all_gather_into_tensor(recv.view(-1), send, group=self.group)
-        idx_all = recv[:, :idx_bytes].contiguous().view(torch.int64).view(world, F, n).permute(1, 0, 2).contiguous()
-        g_all = recv[:, idx_bytes:].contiguous().view(torch.float32).view(world * n, width)
-        total = sum((s.rows * s.dim + 3) // 4 * 4 for s in sources)
-        slab = torch.empty(total, dtype=torch.float32, device=dev)
-        grads, tables, acc = [], [], 0
-        for t, s in enumerate(sources):
-            g = slab[acc:acc + s.rows * s.dim].view(s.rows, s.dim)
-            acc += (s.rows * s.dim + 3) // 4 * 4
-            grads.append(g)
-            tables.append((idx_all[fpos[s.field]].data_ptr(), g_all.data_ptr() + 4 * cols[t], width, g.data_ptr(),
-                           s.rows, world * n, s.dim))
-            s.param._rk_synced = True            # already the global average: allreduce() leaves it alone
-        sparse.direct_reduce_into(tables, dev)
-        self._keep = (idx_all, g_all, recv, send)        # alive until the next step's exchange (stream-ordered use)
-        return grads
 
     def _take(self, n_floats, device, params):
         """A chunk of the table region for one backward's dense gradients (None: allocate normally).  Only for
@@ -230,11 +83,7 @@ class GradientAllReducer:
         (default: each parameter's .grad) lets a CUDA-graph step pass its static tensors.
         Afterwards every parameter's .grad is a view of the reduced buffer."""
         grads = [p.grad for p in self.params] if grads is None else list(grads)
-        synced = [bool(getattr(p, "_rk_synced", False)) for p in self.params]
-        for p in self.params:
-            if getattr(p, "_rk_synced", False):
-                p._rk_synced = False
-        in_slab = [self._in_slab(g) or sy for g, sy in zip(grads, synced)]
+        in_slab = [self._in_slab(g) for g in grads]
         staged = sum(p.numel() for p, s_ in zip(self.params, in_slab) if not s_)
         # the copied gradients sit right below the table region: [n_staging - staged, n_staging + used) is ONE range
         pos = self.n_staging - staged
@@ -258,17 +107,10 @@ class GradientAllReducer:
         for v in zero:
             v.zero_()
         lo = lo // 4 * 4                                       # 16-byte aligned start (a few stale floats ride along)
-        hi = self.n_staging + self._cursor
-        if self.symmetric is not None:
-            lo = lo // 1024 * 1024                             # the peer-memory kernels want whole, aligned vectors per rank
-            hi = lo + (hi - lo + 1023) // 1024 * 1024
-        r = self.flat[lo:hi]
+        r = self.flat[lo:self.n_staging + self._cursor]
         if self._avg is None:
             self._avg = dist.get_backend(self.group) == "nccl"
-        if self.symmetric is not None:
-            self._symmetric_allreduce(r, *self.symmetric)
-            r.mul_(1.0 / self.world_size)
-        elif self._avg:
+        if self._avg:
             dist.all_reduce(r, op=dist.ReduceOp.AVG, group=self.group)
         else:
             dist.all_reduce(r, op=dist.ReduceOp.SUM, group=self.group)

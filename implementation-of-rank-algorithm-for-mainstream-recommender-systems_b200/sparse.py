@@ -10,7 +10,6 @@
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 
 import torch
@@ -46,36 +45,22 @@ def _i64_array(values):
     return (C.c_int64 * max(len(values), 1))(*values)
 
 
-_plan_streams: dict = {}
-PLAN_STREAM_PRIORITY = int(os.environ.get("RANK_B200_PLAN_PRIORITY", "-1"))
-PLAN_ON_SIDE_STREAM = os.environ.get("RANK_B200_PLAN_STREAM", "1") != "0"
+PLAN_ON_SIDE_STREAM = True          # False: plans and reductions run on the caller's stream (timing, debugging)
+_side_streams: dict = {}
 
 
-def _plan_stream(device):
-    """The per-device side stream the occurrence plans are built on (None: build in-stream)."""
+def _side_stream(device, priority):
+    """A per-device side stream of the given priority (None when PLAN_ON_SIDE_STREAM is off).  The occurrence
+    plans are built on the high-priority one (-1): the sort is short and something (the segment reduce) always
+    ends up waiting for it, while the kernels it shares the GPU with (forward / backward of the hot path, the
+    tower) are long.  The one-launch direct reduction runs on the default-priority one (0) when a sorted
+    reduction runs next to it: it depends on the backward kernel only, not on the plan."""
     if not PLAN_ON_SIDE_STREAM:
         return None
-    key = device.index if device.index is not None else torch.cuda.current_device()
-    stream = _plan_streams.get(key)
+    key = (device.index if device.index is not None else torch.cuda.current_device(), priority)
+    stream = _side_streams.get(key)
     if stream is None:
-        # high priority: the sort is short and something (the segment reduce) always ends up waiting for it, while
-        # the kernels it shares the GPU with (forward / backward of the hot path, the tower) are long
-        stream = _plan_streams[key] = torch.cuda.Stream(device=device, priority=PLAN_STREAM_PRIORITY)
-    return stream
-
-
-_direct_streams = {}
-
-
-def _direct_stream(device):
-    """Side stream of the one-launch direct reduction when a sorted reduction runs next to it (its own stream:
-    it depends on the backward kernel only, not on the plan)."""
-    if not PLAN_ON_SIDE_STREAM:
-        return None
-    key = device.index if device.index is not None else torch.cuda.current_device()
-    stream = _direct_streams.get(key)
-    if stream is None:
-        stream = _direct_streams[key] = torch.cuda.Stream(device=device)
+        stream = _side_streams[key] = torch.cuda.Stream(device=device, priority=priority)
     return stream
 
 
@@ -90,8 +75,6 @@ class GradSource:
     field: int           # which plan field's occurrences feed this table
     param: object = None  # the table tensor itself (where a touched-rows gradient is attached)
 
-
-DIRECT_REDUCE = os.environ.get("RANK_B200_DIRECT", "1") != "0"
 
 # ---- opt-in sparse gradients of the replicated tables (SURVEY 8(f) item 3) ---------------------
 # "dense"  : every table receives a dense [V, D] .grad, as the reference's nn.Embedding(sparse=False)
@@ -133,30 +116,6 @@ def _new_slab(n_floats, device, params):
     return torch.empty(n_floats, dtype=torch.float32, device=device)
 
 
-# Data-parallel exchange of per-occurrence gradients (parallel.GradientAllReducer installs it): when every
-# rank's occurrences of a step fit one direct reduction (world x n <= RK_DIRECT_MAX_N), the ranks all-gather
-# their (index, gradient row) pairs — a few hundred KB — and each reduces the WHOLE global batch's occurrences
-# into its dense gradients, instead of reducing its own and all-reducing 13 MB of mostly-zero tables.
-_occurrence_exchange = None
-
-
-def set_occurrence_exchange(fn) -> None:
-    """fn(plan, sources) -> list of dense gradients (already global), or None to reduce locally."""
-    global _occurrence_exchange
-    _occurrence_exchange = fn
-
-
-def direct_reduce_into(tables, dev) -> None:
-    """rk_embgrad_direct_reduce over prepared (idx, g, ld, dw, rows, n, dim) tuples of device pointers."""
-    lib = _lib.load()
-    tabs = (_lib.RkDirectTable * len(tables))()
-    for k, (idx, g, ld, dw, rows, n, dim) in enumerate(tables):
-        tabs[k].idx, tabs[k].g, tabs[k].ld, tabs[k].dw = idx, g, ld, dw
-        tabs[k].rows, tabs[k].n, tabs[k].dim = rows, n, dim
-    rc = lib.rk_embgrad_direct_reduce(tabs, len(tables), _lib.err_flag(dev).data_ptr(), _lib.stream_ptr())
-    _lib.check(rc, "rk_embgrad_direct_reduce")
-
-
 @dataclass
 class TouchedRows:
     """Sparse gradient of one table, sized without a host sync: `capacity = min(occurrences, table rows)`."""
@@ -186,7 +145,9 @@ class OccurrencePlan:
     * longer columns (DIN / BST histories, batches beyond 8192) and padded sequence fields: the stable
       (field, row) order of rk_plan_build, computed here (it depends on the indices only) on a side
       stream while the forward runs, consumed by rk_embgrad_segment_reduce.
-    `direct=False` sorts every field (the order is then available as sorted_keys / perm)."""
+    `direct=None` reduces directly where the field allows it, unless the table gradients are in the touched-rows
+    mode (set_table_gradients), which needs every field sorted; `direct=False` sorts every field (the order is
+    then available as sorted_keys / perm)."""
 
     def __init__(self, indices: list[torch.Tensor], rows: list[int], seq_len=None, live_mode=None, direct=None):
         """`seq_len[f]` (int64 [B]) and `live_mode[f]` (_lib.LIVE_*) mark field f as a padded
@@ -205,7 +166,7 @@ class OccurrencePlan:
         modes_all = [_lib.LIVE_ALL] * self.F if live_mode is None else [int(m) for m in live_mode]
         self.touched = _TABLE_GRADIENTS == "touched" and direct is None
         self._compact = None
-        use_direct = (DIRECT_REDUCE and not self.touched) if direct is None else bool(direct)
+        use_direct = not self.touched if direct is None else bool(direct)
         self.direct = [use_direct and self.n[f] <= _lib.RK_DIRECT_MAX_N and modes_all[f] == _lib.LIVE_ALL
                        for f in range(self.F)]
         # ---- the fields that need the sorted order
@@ -246,7 +207,7 @@ class OccurrencePlan:
         # (a grad-enabled forward that never runs backward); inside a CUDA-graph capture the fork/join is
         # captured.
         main = torch.cuda.current_stream(dev)
-        side = _plan_stream(dev)
+        side = _side_stream(dev, -1)
         self._ws = ws
         if side is None:
             rc = lib.rk_plan_build(idx_ptrs, _i64_array(self.s_n), _i64_array(self.s_rows), S,
@@ -277,10 +238,6 @@ class OccurrencePlan:
         a `touched_grad` and the returned gradients are None."""
         if self.touched:
             return self._reduce_touched(sources)
-        if _occurrence_exchange is not None:
-            done = _occurrence_exchange(self, sources)
-            if done is not None:
-                return done
         lib = _lib.load()
         T = len(sources)
         if not 1 <= T <= _lib.RK_MAX_TABLES:
@@ -321,7 +278,7 @@ class OccurrencePlan:
                 tabs[k].dim = s.dim
             # the two reductions write disjoint parts of the slab: when both exist, the one-launch direct
             # reduction runs on the side stream next to the sorted one (forked and joined here)
-            side = _direct_stream(dev) if n_direct < T else None
+            side = _side_stream(dev, 0) if n_direct < T else None
             if side is None:
                 rc = lib.rk_embgrad_direct_reduce(tabs, n_direct, _lib.err_flag(dev).data_ptr(), _lib.stream_ptr())
             else:

@@ -14,18 +14,16 @@ in training mode on CUDA it runs both modules in one CUDA kernel per direction (
 reading the modules' own parameters and updating their running statistics in place.  Anything
 else (eval mode, other layers, momentum=None, batches below MIN_BATCH or above 16384) runs the modules
 themselves.
-Set `rank_b200.tower.FUSED = False` (or RANK_B200_FUSED_TOWER=0) to always run the modules.
+Set `rank_b200.tower.FUSED = False` to always run the modules.
 """
 from __future__ import annotations
-
-import os
 
 import torch
 import torch.nn as nn
 
 from . import _lib
 
-FUSED = os.environ.get("RANK_B200_FUSED_TOWER", "1") != "0"
+FUSED = True
 # Below this batch size the modules run as they are: batch statistics over a few dozen rows make every
 # gradient a difference of near-equal sums, and the parity bar against the reference (1e-5) is then
 # decided by which fp32 summation order one happens to share with ATen.

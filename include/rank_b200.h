@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RK_ABI_VERSION 2
+#define RK_ABI_VERSION 3
 #define RK_MAX_FIELDS 24
 #define RK_MAX_TABLES 32
 #define RK_MAX_LAYERS 8
@@ -196,12 +196,12 @@ typedef struct rk_din_args {
                                          bf16 operands / fp32 TMEM accumulators (D = 16, 2e-2 bar) */
     const float*        mlp;
     int64_t             B;
-    void*               mlp_tiles;    /* RK_DIN_BF16_TENSOR only, may be NULL: rk_din_tile_bytes() bytes of
+    void*               mlp_tiles;    /* RK_DIN_BF16_TENSOR only, required there: rk_din_tile_bytes() bytes of
                                          scratch (128-byte aligned) that rk_din_fwd fills with the split-bf16
                                          operand tiles of `mlp` for both directions (one small prologue launch);
-                                         every CTA then fetches its weights with one bulk (TMA) copy instead of
-                                         converting them itself.  rk_din_bwd reads what the forward wrote: pass
-                                         the same buffer, untouched in between. */
+                                         every CTA then fetches its weights with one bulk (TMA) copy.
+                                         rk_din_bwd reads what the forward wrote: pass the same buffer,
+                                         untouched in between. */
 } rk_din_args_t;
 #define RK_DIN_FP32 0
 #define RK_DIN_BF16_TENSOR 1
@@ -234,10 +234,10 @@ int rk_afm_bwd(const rk_field_t* fields, int F, const float* w1, const float* b1
                int32_t* err_flag, rk_stream_t stream);
 /* The same forward with the attention MLP on the tensor cores (tcgen05.mma, split-bf16 operands
  * hi.hi + lo.hi + hi.lo, fp32 accumulation in TMEM); same arguments and outputs as rk_afm_fwd, plus
- * `tiles`: NULL, or rk_afm_tile_bytes() bytes of scratch (128-byte aligned) that the forward fills
+ * `tiles` (required): rk_afm_tile_bytes() bytes of scratch (128-byte aligned) that the forward fills
  * once (one small prologue launch) with the weights' operand tiles for BOTH directions; every CTA
- * then fetches them by bulk (TMA) copy instead of converting them itself.  rk_afm_tc_bwd reads
- * what the forward wrote: pass the same buffer, untouched in between (or NULL). */
+ * then fetches them by bulk (TMA) copy.  rk_afm_tc_bwd reads what the forward wrote: pass the
+ * same buffer, untouched in between. */
 int rk_afm_tile_bytes(void);
 int rk_afm_tc_fwd(const rk_field_t* fields, int F, const float* w1, const float* b1, const float* w2,
                   const float* b2, int A, int64_t B, float* out, void* tiles, int32_t* err_flag,
@@ -311,19 +311,15 @@ int rk_rowwise_adam_touched(float* weight, float* exp_avg, float* exp_avg_sq, co
  *   rk_shard_route : given the stable owner-sorted order of owner[] from rk_plan_build
  *                    (sorted_owner, perm), write send_local[i] = owner-local row of the i-th sorted
  *                    request, inv[p] = sorted slot of original position p, counts[w] = requests
- *                    for rank w (W <= 64)
- *   rk_plan_compact: for an all-live single-field plan, rank_keys[i] = number of distinct rows
- *                    before sorted position i, uniq_rows[r] = the r-th distinct row, *n_uniq =
- *                    their count; rk_embgrad_segment_reduce run on rank_keys (rows = *n_uniq)
- *                    then yields the compact [n_uniq, D] gradient of a sparse update. */
+ *                    for rank w (W <= 64) */
 int rk_shard_owner(const int64_t* idx, int64_t n, int64_t rows_total, int64_t rows_per_rank,
                    int64_t* owner, int32_t* err_flag, rk_stream_t stream);
 int rk_shard_route(const int64_t* idx, const uint32_t* sorted_owner, const uint32_t* perm, int64_t n,
                    int64_t rows_total, int64_t rows_per_rank, int W, int64_t* send_local, int64_t* inv,
                    int64_t* counts, rk_stream_t stream);
-int rk_plan_compact(const uint32_t* sorted_keys, int64_t n, int64_t rows, uint32_t* rank_keys,
-                    int64_t* uniq_rows, int64_t* n_uniq, rk_stream_t stream);
-/* The multi-field form, for the touched-rows gradients of replicated tables (SURVEY 8(f) item 3):
+/* Dense ranks of a sorted plan, for the touched-rows gradients of replicated tables (SURVEY 8(f)
+ * item 3): rank_keys[i] = number of distinct rows before sorted position i, so that
+ * rk_embgrad_segment_reduce run on rank_keys yields the compact [distinct rows, D] gradient.
  * sorted_keys is a whole rk_plan_build output over F fields (field f: n[f] keys, rows[f] table
  * rows).  Field f's slice of rank_keys receives keys in the layout rk_embgrad_segment_reduce
  * expects for tables of cap[f] rows (cap[f] >= the number of distinct rows; dead positions are

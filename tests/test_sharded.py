@@ -220,59 +220,3 @@ def test_sharded_bst_two_ranks_nccl(wechat_vocab_dir):
         rank, res = out.get()
         for sparse, (e_logit, e_shard, e_rest) in res.items():
             assert e_logit <= 1e-5 and e_shard <= 1e-5 and e_rest <= 1e-4, (rank, sparse, e_logit, e_shard, e_rest)
-
-
-def _exchange_worker(rank, world, port, vocab_dir, out):
-    """DeepFM, batch 1024 per rank: the occurrence exchange (all-gather of (index, gradient row), one reduction
-    of the global batch on every rank) against the dense all-reduce of the same step."""
-    import torch.nn.functional as F
-    from rank_b200 import synthetic
-    from rank_b200.parallel import GradientAllReducer
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    torch.cuda.set_device(rank)
-    dev = torch.device("cuda", rank)
-    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
-    batch = synthetic.to_device(synthetic.deepfm_batch(1024, seed=50 + rank), dev)
-    grads = {}
-    for mode in ("allreduce", "exchange"):
-        torch.manual_seed(0)
-        model = rank_b200.DeepFM(vocab_dir, embedding_dim=16, dropout_rate=0.0).to(dev).train()
-        reducer = GradientAllReducer(model, occurrence_exchange=(mode == "exchange"))
-        prob = model(batch["category"])[0]
-        F.binary_cross_entropy(prob.squeeze(1), batch["label"]).backward()
-        reducer.allreduce()
-        torch.cuda.synchronize()
-        grads[mode] = {k: p.grad.detach().clone() for k, p in model.named_parameters()}
-        reducer.detach()
-    worst = 0.0
-    for k, g in grads["allreduce"].items():
-        scale = max(float(g.abs().max()), 1e-30)
-        worst = max(worst, float((grads["exchange"][k] - g).abs().max()) / scale)
-    # replicas must hold identical gradients after the exchange
-    flat = torch.cat([g.reshape(-1) for g in grads["exchange"].values()])
-    other = [torch.empty_like(flat) for _ in range(world)]
-    dist.all_gather(other, flat)
-    same = all(torch.equal(o, other[0]) for o in other)
-    rank_b200.check_index_errors()
-    out.put((rank, worst, same))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-@pytest.mark.gpu
-def test_occurrence_exchange_matches_dense_allreduce_two_ranks(wechat_vocab_dir):
-    if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs")
-    ctx = mp.get_context("spawn")
-    out = ctx.SimpleQueue()
-    port = _free_port()
-    procs = [ctx.Process(target=_exchange_worker, args=(r, 2, port, wechat_vocab_dir, out)) for r in range(2)]
-    for p in procs:
-        p.start()
-    for p in procs:
-        p.join(300)
-        assert p.exitcode == 0
-    for _ in range(2):
-        rank, worst, same = out.get()
-        assert worst <= 1e-5, (rank, worst)
-        assert same, rank
