@@ -59,6 +59,14 @@ BST_FP32, BST_BF16_TENSOR = 0, 1
 
 LIVE_ALL, LIVE_PREFIX, LIVE_PREFIX_OR_EMPTY = 0, 1, 2
 
+METRICS_NONFINITE, METRICS_BAD_LABEL, METRICS_BAD_GROUP, METRICS_OVERFLOW, METRICS_NOT_PROB = 1, 2, 4, 8, 16
+
+
+class RkMetricsResult(C.Structure):
+    _fields_ = [("pos", C.c_uint64), ("neg", C.c_uint64), ("u2", C.c_uint64), ("correct", C.c_uint64),
+                ("logloss_sum", C.c_double), ("valid_groups", C.c_uint64), ("uauc_sum", C.c_double)]
+
+
 _P = C.c_void_p
 _I = C.c_int
 _L = C.c_int64
@@ -115,6 +123,9 @@ PROTOTYPES = {
     "rk_din_tile_bytes": (_I, []),
     "rk_din_fwd": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "rk_din_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "rk_metrics_append": (_I, [_P, _P, _P, _L, _P, _P, _P, _L, _L, _P, _P, _P]),
+    "rk_metrics_workspace_bytes": (_Z, [_L, _L]),
+    "rk_metrics_compute": (_I, [_P, _P, _P, _L, _L, _P, _Z, _P, _P]),
 }
 
 _lib = None
@@ -154,7 +165,7 @@ class CallTimer:
     synchronize gives {entry point: (calls, total ms)}."""
 
     NO_KERNEL = ("rk_resunit_pack_floats", "rk_din_mlp_floats", "rk_din_tile_bytes", "rk_afm_bwd_ctas", "rk_afm_tc_bwd_ctas", "rk_afm_tile_bytes", "rk_fwfm_bwd_ctas", "rk_dice_bn_max_batch", "rk_bst_grad_floats", "rk_bst_bwd_ctas", "rk_version", "rk_last_error", "rk_device_sm_count", "rk_launch_count", "rk_debug_spin",
-                 "rk_plan_workspace_bytes", "rk_reduce_workspace_bytes")
+                 "rk_plan_workspace_bytes", "rk_reduce_workspace_bytes", "rk_metrics_workspace_bytes")
 
     def __init__(self):
         self.records = []

@@ -15,6 +15,7 @@
 //     stable scatter with up to 10-bit digits — 6 launches for a 20-bit key space, independent of F.
 #include <string.h>
 #include "common.cuh"
+#include "radix_sort.cuh"
 
 namespace rk {
 
@@ -333,6 +334,43 @@ static int bits_for(int64_t rows_plus_sentinel) {
 }
 static bool is_small(int64_t n, int bits) { return n <= kSmallN && bits <= kSmallMaxBits; }
 static size_t al256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+size_t radix_sort_ws_bytes(int64_t n) {
+    const size_t tiles = (size_t)ceil_div(n > 0 ? n : 1, kSortTile);
+    return 2 * al256((size_t)(n > 0 ? n : 0) * 4) + al256((tiles + 1) * kMaxBins * 4);
+}
+
+int radix_sort_u32(uint32_t* keys, uint32_t* vals, uint32_t* keys_out, uint32_t* vals_out, int64_t n,
+                   int bits, void* ws, cudaStream_t s) {
+    RK_CHECK_ARG(bits >= 1 && bits <= 32 && n >= 0 && n < (1ll << 31), "radix_sort_u32: n=%lld bits=%d",
+                 (long long)n, bits);
+    if (n == 0) return 0;
+    const size_t arr = al256((size_t)n * 4);
+    uint32_t* kT = (uint32_t*)ws;
+    uint32_t* vT = (uint32_t*)((char*)ws + arr);
+    uint32_t* hist = (uint32_t*)((char*)ws + 2 * arr);
+    const int tiles  = (int)ceil_div(n, kSortTile);
+    uint32_t* totals = hist + (size_t)tiles * kMaxBins;
+    const int passes = (bits + 9) / 10;
+    const int dbits  = (bits + passes - 1) / passes;
+    const int bins   = 1 << dbits;
+    uint32_t *kin = keys, *vin = vals;
+    for (int p = 0; p < passes; ++p) {
+        const bool last = p == passes - 1;
+        uint32_t* kout = last ? keys_out : (kin == keys ? kT : keys);
+        uint32_t* vout = last ? vals_out : (vin == vals ? vT : vals);
+        tile_hist_kernel<<<tiles, kSortThreads, 0, s>>>(kin, n, p * dbits, bins, tiles, hist);
+        RK_LAUNCH_CHECK();
+        row_scan_kernel<<<bins, 256, 0, s>>>(hist, tiles, totals);
+        RK_LAUNCH_CHECK();
+        scatter_kernel<<<tiles, kSortThreads, (size_t)kSortWarps * bins * 4, s>>>(
+            kin, vin, kout, vout, n, p * dbits, bins, tiles, hist, totals, 0u);
+        RK_LAUNCH_CHECK();
+        kin = kout;
+        vin = vout;
+    }
+    return 0;
+}
 
 }  // namespace rk
 

@@ -385,6 +385,44 @@ int rk_bst_block_bwd(const rk_bst_block_t* blk, int nhead, const float* table, c
                      float* g_params, float* partials, int n_ctas, int32_t* err_flag,
                      rk_stream_t stream);
 
+/* ---- evaluation metrics (the per-step loss.item()/label.cpu()/prob.cpu() and the per-epoch
+ *      sklearn roc_auc_score / accuracy_score of train()/evaluate(), DeepFM/deepfm.py:173-180,
+ *      :184-208; the challenge's per-user AUC, which the reference cannot compute) -------------
+ * rk_metrics_append copies a batch of B scores / labels (fp32) and, when group != NULL, group ids
+ * (int64) into score_buf / label_buf / group_buf[capacity] at offset count[0], then advances
+ * count[0] (clamped to capacity).  count is int64_t[2]: count[1] is the launch's arrival counter and
+ * must be 0 between launches (zero both to reset).  One launch, no host synchronisation: it may be
+ * captured in a CUDA graph.  Rows past capacity are dropped.  While copying it raises bits of the
+ * sticky *status: */
+#define RK_METRICS_NONFINITE 1u  /* a score is NaN or infinite */
+#define RK_METRICS_BAD_LABEL 2u  /* a label is not 0 or 1 */
+#define RK_METRICS_BAD_GROUP 4u  /* a group id is outside [0, num_groups) */
+#define RK_METRICS_OVERFLOW  8u  /* more rows than capacity were appended */
+#define RK_METRICS_NOT_PROB 16u  /* a score is outside [0, 1] (log loss / accuracy are undefined) */
+int rk_metrics_append(const float* score, const float* label, const int64_t* group, int64_t B,
+                      float* score_buf, float* label_buf, int64_t* group_buf, int64_t capacity,
+                      int64_t num_groups, int64_t* count, uint32_t* status, rk_stream_t stream);
+/* rk_metrics_compute reduces the first n (< 2^31, host value) stored samples into *result (device):
+ *   pos / neg   samples with label 1 / 0;  u2 = 2U, the doubled Mann-Whitney statistic with ties
+ *               counted one half, so AUC = u2 / (2 pos neg) is sklearn's roc_auc_score, exactly;
+ *   correct     samples with (score > 0.5) == label;  logloss_sum = sum of binary cross-entropies,
+ *               each log clamped at -100 (F.binary_cross_entropy), in double, fixed order;
+ *   with group != NULL (num_groups >= 1): the AUC of every group with both classes, summed in
+ *   double in a fixed order (uauc_sum) over the valid_groups such groups.  Ids outside
+ *   [0, num_groups), which rk_metrics_append flags, are counted as group 0.
+ * Every count is an exact integer (2U <= n^2 / 2 fits uint64), so AUC does not depend on the order
+ * of the samples.  ws: rk_metrics_workspace_bytes(n, num_groups) bytes (num_groups 0 without groups). */
+typedef struct rk_metrics_result {
+    uint64_t pos, neg, u2, correct;
+    double   logloss_sum;
+    uint64_t valid_groups;
+    double   uauc_sum;
+} rk_metrics_result_t;
+size_t rk_metrics_workspace_bytes(int64_t n, int64_t num_groups);
+int rk_metrics_compute(const float* score, const float* label, const int64_t* group, int64_t n,
+                       int64_t num_groups, void* ws, size_t ws_bytes, rk_metrics_result_t* result,
+                       rk_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
