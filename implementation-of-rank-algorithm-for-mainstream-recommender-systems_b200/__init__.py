@@ -25,7 +25,7 @@ from .sharded import RowShardedEmbedding, shard_bst_feedid_table
 from .bst import BSTModel, BSTTransformer, leakyrelu, load_vocabulary
 from .staging import PackedBatch
 from .loader import EncodedWechat
-from .optim import RowwiseAdam
+from .optim import Adam, RowwiseAdam
 from .metrics import BinaryMetrics
 
 __all__ = [
@@ -35,5 +35,5 @@ __all__ = [
     "DeepFM", "FwFM", "DCNModel", "cross_layer", "DeepCrossingModel", "residual_unit", "DIN", "Dice", "din_attention", "din_collate_fn", "set_activation_unit_precision",
     "get_activation_unit_precision",
     "AFM", "create_feature_columns", "RowShardedEmbedding", "shard_bst_feedid_table", "BSTModel", "BSTTransformer", "leakyrelu", "load_vocabulary",
-    "PackedBatch", "EncodedWechat", "RowwiseAdam", "BinaryMetrics",
+    "PackedBatch", "EncodedWechat", "Adam", "RowwiseAdam", "BinaryMetrics",
 ]

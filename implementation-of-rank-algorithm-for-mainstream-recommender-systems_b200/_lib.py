@@ -19,6 +19,7 @@ RK_MAX_FIELDS = 24
 RK_MAX_TABLES = 32
 RK_MAX_LAYERS = 8
 RK_DIRECT_MAX_N = 8192
+RK_ADAM_MAX_TENSORS = 64
 ABI_VERSION = 3
 
 
@@ -55,6 +56,13 @@ class RkBstBlock(C.Structure):
 
 
 BST_FP32, BST_BF16_TENSOR = 0, 1
+
+
+class RkAdamTensor(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in (
+        "param", "exp_avg", "exp_avg_sq", "step", "grad", "touched_rows", "touched_values", "touched_count")] + [
+        ("capacity", C.c_int64), ("rows", C.c_int64), ("dim", C.c_int32), ("lr", C.c_float),
+        ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float), ("reserved", C.c_int32)]
 
 
 LIVE_ALL, LIVE_PREFIX, LIVE_PREFIX_OR_EMPTY = 0, 1, 2
@@ -126,6 +134,7 @@ PROTOTYPES = {
     "rk_metrics_append": (_I, [_P, _P, _P, _L, _P, _P, _P, _L, _L, _P, _P, _P]),
     "rk_metrics_workspace_bytes": (_Z, [_L, _L]),
     "rk_metrics_compute": (_I, [_P, _P, _P, _L, _L, _P, _Z, _P, _P]),
+    "rk_adam_step": (_I, [_P, _I, _P, _P]),
 }
 
 _lib = None

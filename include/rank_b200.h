@@ -304,6 +304,37 @@ int rk_rowwise_adam_touched(float* weight, float* exp_avg, float* exp_avg_sq, co
                             int64_t V, float lr, float beta1, float beta2, float eps, int64_t step,
                             int32_t* err_flag, rk_stream_t stream);
 
+/* ---- dense Adam over every parameter in one launch (the reference's optim.Adam(model.parameters(), lr),
+ *      e.g. DCN/dcn.py:246), bit-identical to torch.optim.Adam(fused=True) without weight decay, amsgrad,
+ *      maximize or grad scaling -------------------------------------------------------------------------
+ * Per element, in fp32, with step = *step (the float32 step tensor, already incremented):
+ *   m = fma(b1, m, fma(-b1, g, g));  v = fma(b2, v, fma(-b2, g*g, g*g))
+ *   p -= (lr / (1 - pow(b1, step))) * m / (sqrt(v) / sqrt(1 - pow(b2, step)) + eps)
+ * A tensor's gradient is either dense (grad, [rows, dim]) or a touched-rows gradient: touched_rows
+ * [capacity] distinct rows in ascending order, touched_values [capacity, dim] their gradient rows, of which
+ * the first *touched_count (device, clamped to [0, capacity]) are live.  Every other row takes g = 0, so its
+ * moments decay as in dense Adam, with no dense gradient in memory.  Touched rows outside [0, rows) are
+ * skipped and raise *err_flag (may be NULL).  param / exp_avg / exp_avg_sq / grad are contiguous fp32; lr,
+ * betas and eps are per tensor, so param groups may differ within one launch.  n <= RK_ADAM_MAX_TENSORS
+ * tensors per launch; no host synchronisation, capturable in a CUDA graph. */
+#define RK_ADAM_MAX_TENSORS 64
+typedef struct rk_adam_tensor {
+    float*         param;          /* [rows, dim] */
+    float*         exp_avg;
+    float*         exp_avg_sq;
+    const float*   step;           /* 0-d float32 */
+    const float*   grad;           /* dense gradient, or NULL for a touched-rows gradient */
+    const int64_t* touched_rows;
+    const float*   touched_values;
+    const int64_t* touched_count;  /* NULL for a dense gradient */
+    int64_t        capacity;
+    int64_t        rows;
+    int32_t        dim;
+    float          lr, beta1, beta2, eps;
+    int32_t        reserved;
+} rk_adam_tensor_t;
+int rk_adam_step(const rk_adam_tensor_t* tensors, int n, int32_t* err_flag, rk_stream_t stream);
+
 /* ---- row-sharded table (BASELINE config 5 "scaled": BST feedid table of 1e8 rows block-
  *      partitioned by row over the ranks; the reference itself is single-process) ------------
  * Bookkeeping around the two all-to-alls (indices out / rows back, mirrored for gradients):
