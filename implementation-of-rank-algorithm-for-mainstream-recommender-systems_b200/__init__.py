@@ -25,6 +25,7 @@ from .sharded import RowShardedEmbedding, shard_bst_feedid_table
 from .bst import BSTModel, BSTTransformer, leakyrelu, load_vocabulary
 from .staging import PackedBatch
 from .loader import EncodedWechat
+from .device_data import BatchFeed, DeviceWechat
 from .optim import Adam, RowwiseAdam
 from .metrics import BinaryMetrics
 
@@ -35,5 +36,5 @@ __all__ = [
     "DeepFM", "FwFM", "DCNModel", "cross_layer", "DeepCrossingModel", "residual_unit", "DIN", "Dice", "din_attention", "din_collate_fn", "set_activation_unit_precision",
     "get_activation_unit_precision",
     "AFM", "create_feature_columns", "RowShardedEmbedding", "shard_bst_feedid_table", "BSTModel", "BSTTransformer", "leakyrelu", "load_vocabulary",
-    "PackedBatch", "EncodedWechat", "Adam", "RowwiseAdam", "BinaryMetrics",
+    "PackedBatch", "EncodedWechat", "DeviceWechat", "BatchFeed", "Adam", "RowwiseAdam", "BinaryMetrics",
 ]

@@ -75,6 +75,19 @@ class RkMetricsResult(C.Structure):
                 ("logloss_sum", C.c_double), ("valid_groups", C.c_uint64), ("uauc_sum", C.c_double)]
 
 
+RK_BATCH_MAX_COLS = 32
+BATCH_WINDOW, BATCH_BAD_ROW, BATCH_SEQ_OVERFLOW = 1, 2, 4
+
+
+class RkBatchCol(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("row_bytes", C.c_int64)]
+
+
+class RkBatchSeq(C.Structure):
+    _fields_ = [("values", C.c_void_p), ("offsets", C.c_void_p), ("dst", C.c_void_p), ("dst_len", C.c_void_p),
+                ("width", C.c_int32), ("reserved", C.c_int32)]
+
+
 _P = C.c_void_p
 _I = C.c_int
 _L = C.c_int64
@@ -135,6 +148,7 @@ PROTOTYPES = {
     "rk_metrics_workspace_bytes": (_Z, [_L, _L]),
     "rk_metrics_compute": (_I, [_P, _P, _P, _L, _L, _P, _Z, _P, _P]),
     "rk_adam_step": (_I, [_P, _I, _P, _P]),
+    "rk_batch_gather": (_I, [_P, _I, _P, _P, _L, _L, _P, _L, _L, _P, _P]),
 }
 
 _lib = None

@@ -166,6 +166,13 @@ class EncodedWechat:
             return {k: out[k] for k in ("dense", "category", "seq_feedid", "seq_length", "label")}
         return {k: out[k] for k in ("dense", "category", "label")}
 
+    def to_device(self, device, seq_width=None):
+        """The encoded arrays uploaded once to `device` (plain copies), as a `device_data.DeviceWechat` whose
+        batches are gathered there by one kernel launch each.  `seq_width` (DIN only) is the fixed history
+        width of its graph-capturable feed: at least the longest history, which is the default."""
+        from .device_data import DeviceWechat
+        return DeviceWechat(self, device, seq_width)
+
     def batches(self, batch_size, shuffle=False, generator=None, drop_last=False, packed=None):
         """Iterate over the frame like `DataLoader(dataset, batch_size, shuffle)`.  With `packed`
         (a `PackedBatch` laid out for full batches) every full batch is written into its pinned buffer

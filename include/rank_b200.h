@@ -454,6 +454,40 @@ int rk_metrics_compute(const float* score, const float* label, const int64_t* gr
                        int64_t num_groups, void* ws, size_t ws_bytes, rk_metrics_result_t* result,
                        rk_stream_t stream);
 
+/* ---- batch assembly from an encoded frame in device memory (each script's WechatDataset.__getitem__
+ *      + DataLoader collation: DIN/din.py:86-222 with din_collate_fn, BST/bst.py:94-159,
+ *      DCN/dcn.py:52-112, DeepFM/deepfm.py:26-70) --------------------------------------------------
+ * rk_batch_gather writes one batch of B rows into caller-owned outputs.  Output row i takes source row
+ * r = order[*cursor + row0 + i]: `cursor` is a device int64 the kernel reads, so a captured launch takes
+ * whatever batch the cursor names when it is replayed (advance it in-stream afterwards); row0 is a
+ * data-parallel rank's offset inside the global batch.
+ *   cols[c]: dst row i = the row_bytes bytes of src row r (bytes are copied, never converted);
+ *   seq (may be NULL): the ragged history values[offsets[r] .. offsets[r+1]) written to dst[i, 0..width)
+ *            and zero-padded, its length to dst_len[i] (din_collate_fn's padding).
+ * All columns are one launch; no host synchronisation.  Sticky bits of *status (no fault, and nothing is
+ * written outside the outputs): */
+#define RK_BATCH_MAX_COLS 32
+#define RK_BATCH_WINDOW       1u  /* *cursor < 0 or *cursor + row0 + B > n_order: the batch writes nothing */
+#define RK_BATCH_BAD_ROW      2u  /* an order entry is outside [0, n_rows): that row is written as zeros */
+#define RK_BATCH_SEQ_OVERFLOW 4u  /* a history is longer than width: its first width ids are written and
+                                     its length is written as width */
+typedef struct rk_batch_col {
+    const void* src;        /* [n_rows, row_bytes] */
+    void*       dst;        /* [B, row_bytes] */
+    int64_t     row_bytes;
+} rk_batch_col_t;
+typedef struct rk_batch_seq {
+    const int64_t* values;  /* flat ids of every row's history */
+    const int64_t* offsets; /* [n_rows + 1] */
+    int64_t*       dst;     /* [B, width] */
+    int64_t*       dst_len; /* [B] */
+    int32_t        width;
+    int32_t        reserved;
+} rk_batch_seq_t;
+int rk_batch_gather(const rk_batch_col_t* cols, int n_cols, const rk_batch_seq_t* seq, const int64_t* order,
+                    int64_t n_order, int64_t n_rows, const int64_t* cursor, int64_t row0, int64_t B,
+                    uint32_t* status, rk_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
