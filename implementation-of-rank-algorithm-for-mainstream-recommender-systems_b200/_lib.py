@@ -147,6 +147,7 @@ PROTOTYPES = {
     "rk_metrics_append": (_I, [_P, _P, _P, _L, _P, _P, _P, _L, _L, _P, _P, _P]),
     "rk_metrics_workspace_bytes": (_Z, [_L, _L]),
     "rk_metrics_compute": (_I, [_P, _P, _P, _L, _L, _P, _Z, _P, _P]),
+    "rk_metrics_merge": (_I, [_P, _P, _P, _P, _L, _L, _P, _P, _P, _P, _P]),
     "rk_adam_step": (_I, [_P, _I, _P, _P]),
     "rk_batch_gather": (_I, [_P, _I, _P, _P, _L, _L, _P, _L, _L, _P, _P]),
 }

@@ -20,6 +20,9 @@
 // the run is counted once, by whichever comes later.  NC is a prefix sum and RS / NRS / NGS are
 // "last start" values, i.e. prefix maxima: a tile pass of aggregates, one CTA that scans them, and a
 // tile pass that finishes the scan and adds each group's in-tile segment to that group's counters.
+//
+// Data-parallel ranks: rk_metrics_merge concatenates the all-gathered buffers of every rank (each rank's
+// filled prefix, rank-major) and ORs their statuses, so rk_metrics_compute sees the whole evaluation set.
 #include <string.h>
 #include "common.cuh"
 #include "radix_sort.cuh"
@@ -396,6 +399,61 @@ metrics_final_kernel(const double* __restrict__ ll_part, const unsigned long lon
     }
 }
 
+// ---------------------------------------------------------------------------------------- merge
+// Every CTA copies part of one rank's segment: rank r = blockIdx.x / ctas_per_rank.  It recomputes the
+// segment's offset (the clamped counts of the ranks before r) from the world*3 state words, so the
+// launch needs no scan of its own and no host value of any count.
+constexpr int kMergeThreads = 256;
+constexpr int kMergeMaxCtasPerRank = 1024;
+
+__device__ __forceinline__ int64_t merge_count(const int64_t* state_g, int64_t r, int64_t cap) {
+    const int64_t c = state_g[3 * r];
+    return c < 0 ? 0 : (c > cap ? cap : c);
+}
+
+__global__ void __launch_bounds__(kMergeThreads)
+metrics_merge_kernel(const float* __restrict__ score_g, const float* __restrict__ label_g,
+                     const int64_t* __restrict__ group_g, const int64_t* __restrict__ state_g, int64_t world,
+                     int64_t cap, int64_t ctas_per_rank, float* __restrict__ score_out,
+                     float* __restrict__ label_out, int64_t* __restrict__ group_out, int64_t* __restrict__ state_out) {
+    __shared__ int64_t off_w[kMergeThreads / 32];
+    __shared__ uint32_t bits_w[kMergeThreads / 32];
+    const int64_t r = blockIdx.x / ctas_per_rank, c = blockIdx.x % ctas_per_rank;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    // block 0 sums every rank (the merged count) and ORs every status; the others only the ranks before r
+    const int64_t upto = blockIdx.x == 0 ? world : r;
+    int64_t off = 0;
+    uint32_t bits = 0;
+    for (int64_t q = threadIdx.x; q < upto; q += kMergeThreads) {
+        off += merge_count(state_g, q, cap);
+        bits |= (uint32_t)state_g[3 * q + 2];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) off += __shfl_xor_sync(kFull, off, o);
+    bits = __reduce_or_sync(kFull, bits);
+    if (lane == 0) { off_w[w] = off; bits_w[w] = bits; }
+    __syncthreads();
+    off = 0;
+    bits = 0;
+#pragma unroll
+    for (int k = 0; k < kMergeThreads / 32; ++k) { off += off_w[k]; bits |= bits_w[k]; }
+    if (blockIdx.x == 0) {
+        if (threadIdx.x == 0) {
+            state_out[0] = off;
+            state_out[1] = 0;
+            state_out[2] = (int64_t)bits;
+        }
+        off = 0;   // rank 0's segment starts at 0
+    }
+    const int64_t n_r = merge_count(state_g, r, cap);
+    const int64_t src = r * cap;
+    for (int64_t i = c * kMergeThreads + threadIdx.x; i < n_r; i += ctas_per_rank * kMergeThreads) {
+        score_out[off + i] = score_g[src + i];
+        label_out[off + i] = label_g[src + i];
+        if (group_g) group_out[off + i] = group_g[src + i];
+    }
+}
+
 static size_t al256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 struct MetricsWs {
@@ -509,6 +567,27 @@ int rk_metrics_compute(const float* score, const float* label, const int64_t* gr
     }
     metrics_final_kernel<<<1, kFinalThreads, 0, s>>>(w.ll_part, w.acc_part, tiles, all, G, gu2, gu2 + G,
                                                       gu2 + 2 * G, result);
+    RK_LAUNCH_CHECK();
+    return 0;
+}
+
+int rk_metrics_merge(const float* score_g, const float* label_g, const int64_t* group_g, const int64_t* state_g,
+                     int64_t world, int64_t capacity, float* score_out, float* label_out, int64_t* group_out,
+                     int64_t* state_out, rk_stream_t stream_) {
+    using namespace rk;
+    RK_CHECK_ARG(world >= 1 && capacity >= 1 && world <= ((1ll << 31) - 1) / capacity,
+                 "rk_metrics_merge: world=%lld capacity=%lld (need >= 1 each and world*capacity < 2^31)",
+                 (long long)world, (long long)capacity);
+    RK_CHECK_ARG(score_g && label_g && state_g && score_out && label_out && state_out,
+                 "rk_metrics_merge: NULL buffer");
+    RK_CHECK_ARG(!group_g || group_out, "rk_metrics_merge: group_g needs group_out");
+    RK_CHECK_ARG(state_out + 3 <= state_g || state_out >= state_g + 3 * world,
+                 "rk_metrics_merge: state_out overlaps state_g");
+    const int64_t per = ceil_div(capacity, kMergeThreads);
+    const int64_t ctas_per_rank = per < kMergeMaxCtasPerRank ? per : kMergeMaxCtasPerRank;
+    metrics_merge_kernel<<<(unsigned)(world * ctas_per_rank), kMergeThreads, 0, (cudaStream_t)stream_>>>(
+        score_g, label_g, group_g, state_g, world, capacity, ctas_per_rank, score_out, label_out, group_out,
+        state_out);
     RK_LAUNCH_CHECK();
     return 0;
 }

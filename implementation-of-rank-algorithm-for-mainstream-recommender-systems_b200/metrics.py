@@ -17,6 +17,10 @@ both classes, averaged over those groups.
         metrics.update(prob, batch["label"], batch["category"]["userid"])
     print(metrics.compute())     # {'n', 'auc', 'logloss', 'accuracy', 'uauc'}
     metrics.reset()
+
+Under data parallelism each rank updates with its own shard, and `metrics.all_gather().compute()` gives every
+rank the metrics of all ranks' samples together (one collective per buffer and one merge launch,
+csrc/metrics.cu rk_metrics_merge).
 """
 from __future__ import annotations
 
@@ -58,6 +62,7 @@ class BinaryMetrics:
         self._state = torch.zeros(3, dtype=torch.int64, device=self.device)
         self._result = torch.zeros(_lib.C.sizeof(_lib.RkMetricsResult) // 8, dtype=torch.int64, device=self.device)
         self._ws = None
+        self._gather = None     # (group, world, gather buffers, merged metrics) of all_gather, made on its first call
 
     def reset(self) -> None:
         """Forget every sample and every raised error (enqueued on the current stream)."""
@@ -136,6 +141,63 @@ class BinaryMetrics:
                 raise ValueError("No group has both classes: uAUC is not defined.")
             out["uauc"] = r.uauc_sum / r.valid_groups
         return out
+
+    def all_gather(self, group=None) -> "BinaryMetrics":
+        """The samples of every rank of the process group `group` (default: the world) in one `BinaryMetrics`
+        of capacity world * capacity, whose `compute()` gives the metrics of the whole evaluation set: the
+        single-process result, since AUC and uAUC do not depend on the order of the samples.  The storage
+        order is rank-major (rank 0's samples, then rank 1's, ...).  Every rank of the group must call it.
+
+        The first call is eager: it exchanges (capacity, num_groups) on the host, raises the same ValueError
+        on every rank if they differ, and allocates the gather buffers and the returned object.  Every later
+        call returns that same object and enqueues device work only, on the current stream: one
+        `all_gather_into_tensor` per buffer (scores, labels, groups, state) and one `rk_metrics_merge`
+        launch.  It can be captured in a CUDA graph, e.g. with the last evaluation step.  An error raised on
+        any rank (NaN, a bad label or group id, samples past capacity) travels in the merged status, so
+        `compute()` on the result raises the same ValueError on every rank.
+
+        Without an initialised process group the world is this process alone, and the result's `compute()`
+        equals `self.compute()`."""
+        import torch.distributed as dist
+        lib = _lib.load()
+        distributed = dist.is_available() and dist.is_initialized()
+        if self._gather is None:
+            self._gather = self._gather_setup(group if distributed else None, distributed)
+        elif group is not self._gather[0]:
+            raise ValueError("all_gather: a BinaryMetrics gathers over the group of its first all_gather call")
+        group, world, bufs, merged = self._gather
+        if distributed:
+            for dst, src in zip(bufs, (self.scores, self.labels, self.groups, self._state)):
+                if src is not None:
+                    dist.all_gather_into_tensor(dst, src, group=group)
+        score_g, label_g, group_g, state_g = bufs
+        rc = lib.rk_metrics_merge(score_g.data_ptr(), label_g.data_ptr(), _lib.ptr(group_g), state_g.data_ptr(),
+                                  world, self.capacity, merged.scores.data_ptr(), merged.labels.data_ptr(),
+                                  _lib.ptr(merged.groups), merged._state.data_ptr(), _lib.stream_ptr())
+        _lib.check(rc, "rk_metrics_merge")
+        return merged
+
+    def _gather_setup(self, group, distributed):
+        if not distributed:
+            # world 1: the merge reads this object's own buffers
+            bufs = (self.scores, self.labels, self.groups, self._state)
+            return group, 1, bufs, BinaryMetrics(self.capacity, self.device, self.num_groups)
+        import torch.distributed as dist
+        world = dist.get_world_size(group)
+        mine = torch.tensor([self.capacity, self.num_groups or 0], dtype=torch.int64, device=self.device)
+        every = torch.empty(2 * world, dtype=torch.int64, device=self.device)
+        dist.all_gather_into_tensor(every, mine, group=group)
+        config = [tuple(c) for c in every.view(world, 2).tolist()]
+        if any(c != config[0] for c in config):
+            raise ValueError("all_gather: the ranks' BinaryMetrics differ in (capacity, num_groups or 0): "
+                             + ", ".join(f"rank {r}: {c}" for r, c in enumerate(config)))
+        merged = BinaryMetrics(world * self.capacity, self.device, self.num_groups)   # ValueError past 2^31
+        n = world * self.capacity
+        bufs = (torch.empty(n, dtype=torch.float32, device=self.device),
+                torch.empty(n, dtype=torch.float32, device=self.device),
+                None if self.groups is None else torch.empty(n, dtype=torch.int64, device=self.device),
+                torch.empty(3 * world, dtype=torch.int64, device=self.device))
+        return group, world, bufs, merged
 
 
 def _one_shot(scores, labels, groups=None, num_groups=None) -> dict:

@@ -453,6 +453,18 @@ size_t rk_metrics_workspace_bytes(int64_t n, int64_t num_groups);
 int rk_metrics_compute(const float* score, const float* label, const int64_t* group, int64_t n,
                        int64_t num_groups, void* ws, size_t ws_bytes, rk_metrics_result_t* result,
                        rk_stream_t stream);
+/* rk_metrics_merge joins the buffers of `world` data-parallel ranks, each of the same `capacity`, as an
+ * all-gather lays them out: rank r's samples are score_g / label_g / group_g[r*capacity ...] and its
+ * {count, arrival counter, status} are state_g[3r .. 3r+2].  Rank r's first count_r samples (count_r
+ * clamped to [0, capacity], as rk_metrics_append clamps it) go to score_out / label_out / group_out at
+ * offset count_0 + ... + count_{r-1}, so the storage order is rank-major; state_out gets {sum of the
+ * counts, 0, OR of the statuses}, so rk_metrics_compute on the merged buffers sees every rank's samples and
+ * errors.  group_g may be NULL (then group_out is not written).  Outputs must not overlap the inputs.  One
+ * launch reading the counts on the device, no host synchronisation: it may be captured in a CUDA graph.
+ * Refused before any CUDA call: world or capacity < 1, world*capacity >= 2^31, a NULL required pointer. */
+int rk_metrics_merge(const float* score_g, const float* label_g, const int64_t* group_g, const int64_t* state_g,
+                     int64_t world, int64_t capacity, float* score_out, float* label_out, int64_t* group_out,
+                     int64_t* state_out, rk_stream_t stream);
 
 /* ---- batch assembly from an encoded frame in device memory (each script's WechatDataset.__getitem__
  *      + DataLoader collation: DIN/din.py:86-222 with din_collate_fn, BST/bst.py:94-159,
