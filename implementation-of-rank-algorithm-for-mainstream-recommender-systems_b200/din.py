@@ -30,6 +30,7 @@ SEQ = "his_read_comment_7d_seq"
 SEQ_LEN = "his_read_comment_7d_seq_length"
 
 _PRECISION = "fp32"
+_TC_MAX_T = 128          # widest history of the tensor-core activation unit (fp32 takes any width)
 
 
 def set_activation_unit_precision(mode):
@@ -126,6 +127,10 @@ def _din_args(cat_tables, cat_idx, cat_offsets, dense_cols, target_w, target_idx
         # the tensor-core unit is built for D = 16 (the model's dim): no silent fp32 fallback
         raise _lib.RankB200Error(f"the tcgen05 activation unit needs embedding dim 16, got {int(his_w.shape[1])}; "
                                  "use precision 'fp32' for other dims")
+    if precision == "bf16" and a.T > _TC_MAX_T:
+        # the tensor-core unit packs whole histories into 128-row tiles: no silent fp32 fallback either
+        raise _lib.RankB200Error(f"the tcgen05 activation unit takes histories of at most {_TC_MAX_T} positions, "
+                                 f"got {a.T}; use precision 'fp32' for longer ones")
     a.precision = 1 if precision == "bf16" else 0
     mlp = _lib.require_cuda(mlp, "attention mlp", torch.float32)
     if mlp.numel() != _lib.load().rk_din_mlp_floats(int(hw.shape[1])):
@@ -172,6 +177,8 @@ class _DinHotPath(torch.autograd.Function):
             idx_cols = [keep[1][2 * f + 1] for f in range(F)] + [keep[5], keep[7]]
             rows = [int(t.shape[0]) for t in cat_tabs] + [int(tgt_w.shape[0]), int(his_w.shape[0])]
             mode = _lib.LIVE_PREFIX_OR_EMPTY if use_softmax else _lib.LIVE_PREFIX
+            if T == 0:
+                mode = _lib.LIVE_ALL      # no positions at all: nothing to mask
             plan = OccurrencePlan(idx_cols, rows, seq_len=[None] * (F + 1) + [keep[8]],
                                   live_mode=[_lib.LIVE_ALL] * (F + 1) + [mode])
         rc = lib.rk_din_fwd(C.byref(a), concat_all.data_ptr(), norm.data_ptr(), att_w.data_ptr(),
@@ -204,7 +211,8 @@ class _DinHotPath(torch.autograd.Function):
         g_concat = None if g_concat is None else _lib.require_cuda(g_concat, "g_concat", torch.float32)
         g_norm = None if g_norm is None else _lib.require_cuda(g_norm, "g_norm", torch.float32)
         g_row = torch.empty(B, width, dtype=torch.float32, device=dev)
-        g_hist = torch.empty(B, T, D, dtype=torch.float32, device=dev)
+        # never a NULL pointer, even with T == 0: the reduction takes the history gradient's address
+        g_hist = torch.empty(max(B * T * D, 1), dtype=torch.float32, device=dev)[:B * T * D].view(B, T, D)
         rc = lib.rk_din_bwd(C.byref(ctx.args), concat_all.data_ptr(), norm.data_ptr(), att_w.data_ptr(),
                             masks.data_ptr(), _lib.ptr(g_concat), _lib.ptr(g_norm), g_row.data_ptr(),
                             g_hist.data_ptr(), _lib.err_flag(dev).data_ptr(), _lib.stream_ptr())

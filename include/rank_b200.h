@@ -208,6 +208,11 @@ typedef struct rk_din_args {
 int rk_din_tile_bytes(void);
 
 int rk_din_mlp_floats(int D);
+/* History width T: any T >= 0 with RK_DIN_FP32.  Up to 128 positions a tile holds whole samples; wider
+ * histories are walked by the same CTAs in chunks of at most 128 rows (raw pooling and the softmax's running
+ * max / sum carried across chunks in a fixed order: deterministic, no atomics, no host synchronisation).
+ * T = 0 (every history empty) gives an attention output of 0 and needs no att_w / relu_masks / history
+ * pointers.  RK_DIN_BF16_TENSOR takes 0 <= T <= 128 and refuses wider histories: use RK_DIN_FP32 there. */
 int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float* att_w,
                uint32_t* relu_masks, int32_t* err_flag, rk_stream_t stream);
 /* g_row[B,width]: per-occurrence gradients of every concat column (tower gradient g_concat + L2
