@@ -42,6 +42,7 @@ _PARAM_ORDER = ("position_embedding.weight", "w_q.weight", "w_q.bias", "w_k.weig
 _FIELD_ORDER = ("pos", "wq", "bq", "wk", "bk", "wv", "bv", "wo", "bo", "ln1_g", "ln1_b", "w1", "b1", "w2", "b2",
                 "ln2_g", "ln2_b")
 _PRECISION = "fp32"
+_TC_MAX_T = 128          # longest sequence of the tensor-core block (fp32 takes any length)
 
 
 def set_block_precision(precision: str) -> None:
@@ -86,6 +87,14 @@ def _block_struct(params, dropout_p, rng, precision):
     return blk, keep
 
 
+def _check_length(T, precision):
+    """The tensor-core block tiles whole sequences into 128 rows: refused above that, before any launch
+    (no silent fp32 fallback)."""
+    if precision == "bf16" and T > _TC_MAX_T:
+        raise _lib.RankB200Error(f"the tcgen05 BST block takes sequences of at most {_TC_MAX_T} positions, "
+                                 f"got {T}; use block precision 'fp32' for longer ones")
+
+
 class _BstBlock(torch.autograd.Function):
     """One transformer block.  source = table (with idx) for the first block, else x[B,T,16].
     Returns y[B,T,16], or the pooled [B,16] when `pool` is 'sum' / 'mean'."""
@@ -106,6 +115,7 @@ class _BstBlock(torch.autograd.Function):
             raise RuntimeError(f"shape '[{B}, {T}, {nhead}, -1]' is invalid for d_model {source.shape[-1]}")
         if params[0].shape[0] < T:
             raise IndexError("index out of range in self")      # position_embedding(arange(T))
+        _check_length(T, precision)
         blk, keep = _block_struct(params, dropout_p, rng, precision)
         dev = source.device
         y = pooled = None
@@ -222,13 +232,17 @@ class BSTTransformer(nn.Module):
         self._last_rng = snap          # what this forward's masks were drawn from (tests read it)
         return p, snap
 
+    def resolve_precision(self, precision=None):
+        """The block precision of a call: `precision`, else this block's, else set_block_precision's."""
+        return precision or getattr(self, "block_precision", None) or _PRECISION
+
     def run(self, source, seq_len, idx=None, pool=None, precision=None):
         """Fused path used by BSTModel: rows from `source[idx]` (first block) or `source[B,T,16]`.
         precision: "fp32" / "bf16" for this call, None = set_block_precision's global setting."""
         if self.d_model != D_MODEL:
             raise NotImplementedError(f"the fused BST block is built for d_model = {D_MODEL}")
         p, rng = self._dropout_state(source.device)
-        precision = precision or getattr(self, "block_precision", None) or _PRECISION
+        precision = self.resolve_precision(precision)
         return _BstBlock.apply((self.nhead, pool, p, rng, precision), seq_len, idx, source, *self._params())
 
     def forward(self, queries, keys, values, key_padding_mask=None):
@@ -280,6 +294,8 @@ class BSTModel(nn.Module):
 
     def hot_path(self, dense, category, seq_feedid, seq_length):
         """The part of forward that runs in librank_b200: (side features [B,50], pooled sequence [B,16])."""
+        for block in self.transformer_blocks:
+            _check_length(int(seq_feedid.shape[1]), block.resolve_precision(self.block_precision))
         cols = [c for c in self.embeddings if c in category]
         side = GatherConcat.apply(len(cols), dense, *[category[c] for c in cols],
                                   *[self.embeddings[c].weight for c in cols])

@@ -383,7 +383,10 @@ int rk_resunits_bwd(const float* nets, const float* units, int n_units, int H, i
  *      :238-241), d_model = 16, nhead in {1,2,4,8,16} ------------------------------------------
  * Input rows x[b,t,:] come either from a table through idx[B,T] (first block: the feedid
  * embedding) or from x_in[B,T,16] (a previous block's output).  Keys t >= seq_len[b] are masked
- * with -inf (a length-0 sample yields NaN, as in the reference).  y_out[B,T,16] and/or the
+ * with -inf (a length-0 sample yields NaN, as in the reference).
+ * Sequence length T: RK_BST_FP32 takes any T >= 1 (above 128 positions a CTA owns one sample at a time and
+ * walks it in 128-row query and key chunks); RK_BST_BF16_TENSOR takes 1 <= T <= 128 and refuses a longer
+ * sequence with an argument error before any CUDA call.  y_out[B,T,16] and/or the
  * pooled row sum_t y[b,t,:] (divided by seq_len[b] when pool_mean) written to
  * pool_out[b*pool_ld + 0..15] are produced.
  * Dropout (BST/bst.py:86 on w_o's output, :62 inside the FFN, :90 on the FFN output): dropout_p > 0
@@ -414,7 +417,8 @@ int rk_bst_block_fwd(const rk_bst_block_t* blk, int nhead, const float* table, c
 /* g_y[B,T,16] and/or g_pool (row b at g_pool + b*g_pool_ld) -> g_x[B,T,16] and the gradients of the
  * block's registered tensors in g_params, laid out
  *   [pos T*16][wq 256][bq 16][wk][bk][wv][bv][wo][bo][ln1_g][ln1_b][w1][b1][w2][b2][ln2_g][ln2_b];
- * partials: scratch of rk_bst_bwd_ctas(B,T,blk->precision) * rk_bst_grad_floats(T) floats. */
+ * partials: scratch of rk_bst_bwd_ctas(B,T,blk->precision) * rk_bst_grad_floats(T) floats (for T > 128 at most
+ * 2^26 floats in all). */
 int rk_bst_block_bwd(const rk_bst_block_t* blk, int nhead, const float* table, const int64_t* idx,
                      int64_t table_rows, const float* x_in, const int64_t* seq_len, int64_t B, int T,
                      const float* g_y, const float* g_pool, int g_pool_ld, int pool_mean, float* g_x,
