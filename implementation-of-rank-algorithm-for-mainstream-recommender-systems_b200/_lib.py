@@ -88,6 +88,19 @@ class RkBatchSeq(C.Structure):
                 ("width", C.c_int32), ("reserved", C.c_int32)]
 
 
+ENCODE_TABLE_FULL, ENCODE_SPLIT_COUNT = 1, 2
+
+
+class RkVocab(C.Structure):
+    _fields_ = [("bytes", C.c_void_p), ("offsets", C.c_void_p), ("pos", C.c_void_p), ("slots", C.c_void_p),
+                ("n_keys", C.c_int64), ("n_slots", C.c_int64)]
+
+
+class RkStrCol(C.Structure):
+    _fields_ = [("bytes", C.c_void_p), ("offsets", C.c_void_p), ("valid", C.c_void_p), ("valid_bit0", C.c_int64),
+                ("n", C.c_int64)]
+
+
 _P = C.c_void_p
 _I = C.c_int
 _L = C.c_int64
@@ -150,6 +163,11 @@ PROTOTYPES = {
     "rk_metrics_merge": (_I, [_P, _P, _P, _P, _L, _L, _P, _P, _P, _P, _P]),
     "rk_adam_step": (_I, [_P, _I, _P, _P]),
     "rk_batch_gather": (_I, [_P, _I, _P, _P, _L, _L, _P, _L, _L, _P, _P]),
+    "rk_vocab_slots": (_L, [_L]),
+    "rk_vocab_build": (_I, [_P, _P, _P]),
+    "rk_encode_strings": (_I, [_P, _P, _P, _L, _P, _P]),
+    "rk_encode_split_count": (_I, [_P, _P, _P]),
+    "rk_encode_split": (_I, [_P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None
@@ -189,7 +207,7 @@ class CallTimer:
     synchronize gives {entry point: (calls, total ms)}."""
 
     NO_KERNEL = ("rk_resunit_pack_floats", "rk_din_mlp_floats", "rk_din_tile_bytes", "rk_afm_bwd_ctas", "rk_afm_tc_bwd_ctas", "rk_afm_tile_bytes", "rk_fwfm_bwd_ctas", "rk_dice_bn_max_batch", "rk_bst_grad_floats", "rk_bst_bwd_ctas", "rk_version", "rk_last_error", "rk_device_sm_count", "rk_launch_count", "rk_debug_spin",
-                 "rk_plan_workspace_bytes", "rk_reduce_workspace_bytes", "rk_metrics_workspace_bytes")
+                 "rk_vocab_slots", "rk_plan_workspace_bytes", "rk_reduce_workspace_bytes", "rk_metrics_workspace_bytes")
 
     def __init__(self):
         self.records = []

@@ -60,10 +60,73 @@ def encode_column(values: pd.Series, index: dict) -> np.ndarray:
     return mapped.fillna(0).to_numpy(dtype=np.int64)
 
 
+def category_columns(kind):
+    """The `category` dict's columns of a batch of this kind."""
+    return SIX if kind == "deepfm" else SIDE
+
+
 def _float_column(frame, col, n):
     if col not in frame.columns:                    # row.get(col, 0.0)
         return np.zeros(n, dtype=np.float32)
     return frame[col].to_numpy(dtype=np.float64).astype(np.float32)   # torch.tensor(float64 value, dtype=float32)
+
+
+def read_frame(data):
+    """The DataFrame itself, or the parquet file at the path `data` read with pandas."""
+    return pd.read_parquet(data) if isinstance(data, (str, os.PathLike)) else data
+
+
+def encode_category(frame, col, index):
+    """One categorical column encoded (`row.get(col)` is None for an absent column: every value unknown)."""
+    if col not in frame.columns:
+        return np.zeros(len(frame), dtype=np.int64)
+    return encode_column(frame[col], index)
+
+
+def din_history(frame, index):
+    """Ragged encoding of `his_read_comment_7d_seq`: flat ids + offsets [N+1] (DIN/din.py:146-158)."""
+    n = len(frame)
+    if DIN_SEQ not in frame.columns:                # row.get(col, []) -> empty history
+        return np.zeros(0, dtype=np.int64), np.zeros(n + 1, dtype=np.int64)
+    col = frame[DIN_SEQ]
+    is_str = col.map(lambda v: isinstance(v, str)).to_numpy(dtype=bool)
+    lists = col.astype(object)                      # (an Arrow-backed string column cannot hold lists)
+    if is_str.any():
+        lists[is_str] = pd.Series([v.split(",") for v in col[is_str]], index=col.index[is_str], dtype=object)
+    bad = [type(v).__name__ for v in lists[~is_str] if not hasattr(v, "__iter__")]
+    if bad:                                         # the reference iterates the value: a float NaN raises there too
+        raise TypeError(f"'{bad[0]}' object is not iterable")
+    lengths = lists.map(len).to_numpy(dtype=np.int64)
+    offsets = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(lengths, out=offsets[1:])
+    flat = lists.explode()
+    keep = np.repeat(lengths > 0, np.maximum(lengths, 1))     # explode keeps one NaN row per empty list
+    items = flat.to_numpy(dtype=object)[keep]
+    ids = pd.Series(items, dtype=object).map(index).fillna(0).to_numpy(dtype=np.int64) if len(items) else \
+        np.zeros(0, dtype=np.int64)
+    return ids, offsets
+
+
+def bst_sequence(frame, index, T):
+    """`feedid` as a sequence cut / padded to T = max_seq_length, and its lengths (BST/bst.py:139-148)."""
+    n = len(frame)
+    seq = np.zeros((n, T), dtype=np.int64)
+    if "feedid" not in frame.columns:               # row.get("feedid", []) -> empty list
+        return seq, np.zeros(n, dtype=np.int64)
+    col = frame["feedid"]
+    is_list = col.map(lambda v: isinstance(v, list)).to_numpy(dtype=bool)
+    length = np.ones(n, dtype=np.int64)
+    if (~is_list).any():
+        seq[~is_list, 0] = encode_column(col[~is_list], index) if T > 0 else 0
+    for row in np.nonzero(is_list)[0]:              # real python lists are rare (parquet yields arrays): plain loop
+        items = col.iloc[row][:T]
+        length[row] = len(items)
+        if items:
+            seq[row, :len(items)] = encode_column(pd.Series(items, dtype=object), index)
+    length = np.minimum(length, T)
+    if T == 0:
+        seq = seq[:, :0]
+    return seq, length
 
 
 class EncodedWechat:
@@ -72,70 +135,21 @@ class EncodedWechat:
     def __init__(self, data, vocab_dir, kind, max_seq_length=50):
         if kind not in KINDS:
             raise ValueError(f"kind must be one of {KINDS}, got {kind!r}")
-        frame = pd.read_parquet(data) if isinstance(data, (str, os.PathLike)) else data
+        frame = read_frame(data)
         self.kind, self.n, self.max_seq_length = kind, len(frame), max_seq_length
         vocab = {c: load_vocab_index(vocab_dir, f) for c, f in VOCAB_FILES.items()}
         self.label = _float_column(frame, "read_comment", self.n)
-        cat_cols = SIX if kind == "deepfm" else SIDE
-        self.category = {c: self._cat(frame, c, vocab[c]) for c in cat_cols}
+        self.category = {c: encode_category(frame, c, vocab[c]) for c in category_columns(kind)}
         if kind != "deepfm":
             self.dense = np.stack([_float_column(frame, c, self.n) for c in DENSE_FEATURES], axis=1)
         if kind == "din":
-            self.target = {"feedid": self._cat(frame, "feedid", vocab["feedid"])}
-            self.seq_flat, self.seq_offsets = self._din_history(frame, vocab["feedid"])
+            self.target = {"feedid": encode_category(frame, "feedid", vocab["feedid"])}
+            self.seq_flat, self.seq_offsets = din_history(frame, vocab["feedid"])
         if kind == "bst":
-            self.seq, self.seq_length = self._bst_sequence(frame, vocab["feedid"])
+            self.seq, self.seq_length = bst_sequence(frame, vocab["feedid"], max_seq_length)
 
     def __len__(self):
         return self.n
-
-    def _cat(self, frame, col, index):
-        if col not in frame.columns:                # row.get(col) is None -> unknown
-            return np.zeros(self.n, dtype=np.int64)
-        return encode_column(frame[col], index)
-
-    def _din_history(self, frame, index):
-        """Ragged encoding of `his_read_comment_7d_seq`: flat ids + offsets [N+1] (DIN/din.py:146-158)."""
-        if DIN_SEQ not in frame.columns:            # row.get(col, []) -> empty history
-            return np.zeros(0, dtype=np.int64), np.zeros(self.n + 1, dtype=np.int64)
-        col = frame[DIN_SEQ]
-        is_str = col.map(lambda v: isinstance(v, str)).to_numpy(dtype=bool)
-        lists = col.astype(object)                  # (an Arrow-backed string column cannot hold lists)
-        if is_str.any():
-            lists[is_str] = pd.Series([v.split(",") for v in col[is_str]], index=col.index[is_str], dtype=object)
-        bad = [type(v).__name__ for v in lists[~is_str] if not hasattr(v, "__iter__")]
-        if bad:                                     # the reference iterates the value: a float NaN raises there too
-            raise TypeError(f"'{bad[0]}' object is not iterable")
-        lengths = lists.map(len).to_numpy(dtype=np.int64)
-        offsets = np.zeros(self.n + 1, dtype=np.int64)
-        np.cumsum(lengths, out=offsets[1:])
-        flat = lists.explode()
-        keep = np.repeat(lengths > 0, np.maximum(lengths, 1))     # explode keeps one NaN row per empty list
-        items = flat.to_numpy(dtype=object)[keep]
-        ids = pd.Series(items, dtype=object).map(index).fillna(0).to_numpy(dtype=np.int64) if len(items) else \
-            np.zeros(0, dtype=np.int64)
-        return ids, offsets
-
-    def _bst_sequence(self, frame, index):
-        """`feedid` as a sequence cut / padded to max_seq_length (BST/bst.py:139-148)."""
-        T = self.max_seq_length
-        seq = np.zeros((self.n, T), dtype=np.int64)
-        if "feedid" not in frame.columns:           # row.get("feedid", []) -> empty list
-            return seq, np.zeros(self.n, dtype=np.int64)
-        col = frame["feedid"]
-        is_list = col.map(lambda v: isinstance(v, list)).to_numpy(dtype=bool)
-        length = np.ones(self.n, dtype=np.int64)
-        if (~is_list).any():
-            seq[~is_list, 0] = encode_column(col[~is_list], index) if T > 0 else 0
-        for row in np.nonzero(is_list)[0]:          # real python lists are rare (parquet yields arrays): plain loop
-            items = col.iloc[row][:T]
-            length[row] = len(items)
-            if items:
-                seq[row, :len(items)] = encode_column(pd.Series(items, dtype=object), index)
-        length = np.minimum(length, T)
-        if T == 0:
-            seq = seq[:, :0]
-        return seq, length
 
     # ------------------------------------------------------------------ batches
     def batch(self, rows):

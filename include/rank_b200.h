@@ -509,6 +509,51 @@ int rk_batch_gather(const rk_batch_col_t* cols, int n_cols, const rk_batch_seq_t
                     int64_t n_order, int64_t n_rows, const int64_t* cursor, int64_t row0, int64_t B,
                     uint32_t* status, rk_stream_t stream);
 
+/* ---- frame encoding on the device (rank_b200.loader.EncodedWechat's encode_column and DIN's history
+ *      split, i.e. each script's vocabulary dict lookup per value: DIN/din.py:146-158, BST/bst.py:139-148,
+ *      DCN/dcn.py:52-112, DeepFM/deepfm.py:26-70) ---------------------------------------------------------
+ * A vocabulary is its n_keys unique keys (UTF-8 bytes[offsets[k] .. offsets[k+1]), each encoding to pos[k])
+ * and an open-addressing table of n_slots 64-bit slots, a power of two >= 2 * n_keys (rk_vocab_slots gives
+ * the smallest), which rk_vocab_build fills.  A string column is Arrow's large_string layout: row i is
+ * bytes[offsets[i] .. offsets[i+1]), null when bit valid_bit0 + i of the LSB-first bitmap `valid` is 0
+ * (valid may be NULL: no nulls).  Values are compared byte for byte.  Argument errors are refused before any
+ * CUDA call; no entry point allocates or synchronises.  Sticky bits of *status (no fault): */
+#define RK_ENCODE_TABLE_FULL  1u  /* a probe visited every slot without finding the key or an empty slot (the
+                                     slots are not a table rk_vocab_build made): the key is not inserted, the
+                                     value encodes to 0 */
+#define RK_ENCODE_SPLIT_COUNT 2u  /* a row's item count differs from out_offsets: items past its range are
+                                     not written */
+typedef struct rk_vocab {
+    const char*    bytes;
+    const int64_t* offsets;  /* [n_keys + 1] */
+    const int64_t* pos;      /* [n_keys] */
+    uint64_t*      slots;    /* [n_slots] */
+    int64_t        n_keys;   /* < 2^31 - 1 */
+    int64_t        n_slots;
+} rk_vocab_t;
+typedef struct rk_str_col {
+    const char*    bytes;
+    const int64_t* offsets;  /* [n + 1] */
+    const uint8_t* valid;    /* may be NULL */
+    int64_t        valid_bit0;
+    int64_t        n;
+} rk_str_col_t;
+/* The smallest power of two >= 2 * n_keys (at least 1); -1 for n_keys < 0 or >= 2^31 - 1. */
+int64_t rk_vocab_slots(int64_t n_keys);
+/* Sets every slot empty, then inserts every key (one thread per key, atomicCAS on a slot, linear probing). */
+int rk_vocab_build(const rk_vocab_t* vocab, uint32_t* status, rk_stream_t stream);
+/* out[i * out_stride] = pos of the key equal to row i, or 0 when there is none or the row is null
+ * (encode_column).  out_stride >= 1, so a column of a wider row-major matrix is written in place. */
+int rk_encode_strings(const rk_vocab_t* vocab, const rk_str_col_t* col, int64_t* out, int64_t out_stride,
+                      uint32_t* status, rk_stream_t stream);
+/* DIN's history split on ',' (str.split(",")), in two passes.  rk_encode_split_count: counts[i] = 1 + the
+ * number of ',' bytes of row i ('' is one item, 'a,' two).  rk_encode_split: item k of row i, encoded as
+ * rk_encode_strings encodes a value, to out[out_offsets[i] + k]; out_offsets is the exclusive scan of the
+ * counts ([n + 1]).  Both ignore `valid` (a null history is refused by the caller, as the reference raises). */
+int rk_encode_split_count(const rk_str_col_t* col, int64_t* counts, rk_stream_t stream);
+int rk_encode_split(const rk_vocab_t* vocab, const rk_str_col_t* col, const int64_t* out_offsets, int64_t* out,
+                    uint32_t* status, rk_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
