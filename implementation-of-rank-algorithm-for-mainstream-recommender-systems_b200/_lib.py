@@ -141,6 +141,8 @@ PROTOTYPES = {
     "rk_dice_bn_bwd": (_I, [_P, _P, _L, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "rk_bn_act_fwd": (_I, [_P, _L, _I, _P, _P, _F, _F, _P, _P, _P, _F, _P, _P, _P]),
     "rk_bn_act_bwd": (_I, [_P, _P, _L, _I, _P, _P, _F, _P, _P, _P, _P, _P]),
+    "rk_linear_wgrad_scratch_floats": (_L, [_L, _I, _I]),
+    "rk_linear_wgrad": (_I, [_P, _L, _P, _L, _L, _I, _I, _P, _P, _P, _P]),
     "rk_rowwise_adam": (_I, [_P, _P, _P, _P, _P, _L, _I, _L, _F, _F, _F, _F, _L, _P, _P]),
     "rk_shard_owner": (_I, [_P, _L, _L, _L, _P, _P, _P]),
     "rk_shard_route": (_I, [_P, _P, _P, _L, _L, _L, _I, _P, _P, _P, _P]),
@@ -207,7 +209,7 @@ class CallTimer:
     synchronize gives {entry point: (calls, total ms)}."""
 
     NO_KERNEL = ("rk_resunit_pack_floats", "rk_din_mlp_floats", "rk_din_tile_bytes", "rk_afm_bwd_ctas", "rk_afm_tc_bwd_ctas", "rk_afm_tile_bytes", "rk_fwfm_bwd_ctas", "rk_dice_bn_max_batch", "rk_bst_grad_floats", "rk_bst_bwd_ctas", "rk_version", "rk_last_error", "rk_device_sm_count", "rk_launch_count", "rk_debug_spin",
-                 "rk_vocab_slots", "rk_plan_workspace_bytes", "rk_reduce_workspace_bytes", "rk_metrics_workspace_bytes")
+                 "rk_vocab_slots", "rk_linear_wgrad_scratch_floats", "rk_plan_workspace_bytes", "rk_reduce_workspace_bytes", "rk_metrics_workspace_bytes")
 
     def __init__(self):
         self.records = []

@@ -19,6 +19,7 @@ import torch.nn as nn
 from . import _lib
 from .ephemeral import EphemeralBuffer
 from .sparse import GradSource, OccurrencePlan, field_array
+from .tower import run_tower
 from .vocab import table_heights
 
 SIDE_COLUMNS = ("userid", "feedid", "device", "authorid", "bgm_song_id", "bgm_singer_id",
@@ -189,7 +190,7 @@ class DCNModel(nn.Module):
 
     def forward(self, dense, category):
         concat_all, cross_vec = self.hot_path(dense, category)
-        dnn_vec = self.dnn(concat_all)
+        dnn_vec = run_tower(list(self.dnn), concat_all)      # = self.dnn(concat_all), Linear weight gradients in librank
         logit = self.output_layer(torch.cat([cross_vec, dnn_vec], dim=1))
         probability = torch.sigmoid(logit)
         return probability, logit

@@ -11,8 +11,10 @@ or
     nn.BatchNorm1d(units) -> nn.ReLU() | nn.LeakyReLU(slope)    (DeepFM/deepfm.py:100-110, BST/bst.py:203-214)
 
 in training mode on CUDA it runs both modules in one CUDA kernel per direction (csrc/tower.cu),
-reading the modules' own parameters and updating their running statistics in place.  Anything
-else (eval mode, other layers, momentum=None, batches below MIN_BATCH or above 16384) runs the modules
+reading the modules' own parameters and updating their running statistics in place.  An nn.Linear
+with at least LINEAR_MIN_OUT outputs keeps torch's forward and input gradient, and takes its weight
+and bias gradients from one csrc/linear.cu call.  Anything else (eval mode, other layers,
+momentum=None, batches below MIN_BATCH, or above 16384 for the normalisation pairs) runs the modules
 themselves.
 Set `rank_b200.tower.FUSED = False` to always run the modules.
 """
@@ -20,6 +22,7 @@ from __future__ import annotations
 
 import torch
 import torch.nn as nn
+import torch.nn.functional as F
 
 from . import _lib
 
@@ -28,6 +31,9 @@ FUSED = True
 # gradient a difference of near-equal sums, and the parity bar against the reference (1e-5) is then
 # decided by which fp32 summation order one happens to share with ATen.
 MIN_BATCH = 256
+# A Linear with fewer outputs than one 64-wide dW tile of csrc/linear.cu keeps torch's weight gradient: the
+# tile is then mostly padding (BST's final Linear(128, 1) at B = 8192: 28 µs against torch's 10 µs).
+LINEAR_MIN_OUT = 64
 
 
 class _DiceBn(torch.autograd.Function):
@@ -111,6 +117,42 @@ class _BnAct(torch.autograd.Function):
         return g_x, g_par[0], g_par[1], None, None
 
 
+def _rows(t):
+    """t with unit column stride, and its row pitch: the kernel reads strided rows in place."""
+    B, n = t.shape
+    if (n > 1 and t.stride(1) != 1) or (B > 1 and t.stride(0) < n):
+        t = t.contiguous()
+    return t, (t.stride(0) if B > 1 else n)
+
+
+class _Linear(torch.autograd.Function):
+    """nn.Linear with torch's forward and input gradient; dW = g^T x and db = sum_b g in one csrc/linear.cu
+    call (cuBLAS runs these as a split-K sgemm over a few dozen output tiles plus a separate bias reduce)."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        ctx.save_for_backward(x, weight)
+        ctx.has_bias = bias is not None
+        return F.linear(x, weight, bias)
+
+    @staticmethod
+    def backward(ctx, g):
+        lib = _lib.load()
+        x, weight = ctx.saved_tensors
+        g_x = g.mm(weight) if ctx.needs_input_grad[0] else None
+        B, K = x.shape
+        N = weight.shape[0]
+        x, ldx = _rows(x)
+        g, ldg = _rows(g)
+        g_w = torch.empty_like(weight)
+        g_b = torch.empty(N, dtype=torch.float32, device=g.device) if ctx.has_bias else None
+        partials = torch.empty(lib.rk_linear_wgrad_scratch_floats(B, K, N), dtype=torch.float32, device=g.device)
+        rc = lib.rk_linear_wgrad(x.data_ptr(), ldx, g.data_ptr(), ldg, B, K, N, g_w.data_ptr(), _lib.ptr(g_b),
+                                 partials.data_ptr() if partials.numel() else None, _lib.stream_ptr())
+        _lib.check(rc, "rk_linear_wgrad")
+        return g_x, g_w, g_b
+
+
 def _activation_slope(layer):
     if type(layer) is nn.ReLU:
         return 0.0
@@ -126,7 +168,7 @@ def _fusable_bn(bn):
 
 def run_tower(layers, x):
     """`for layer in layers: x = layer(x)` with Dice(+BatchNorm1d) and BatchNorm1d+(Leaky)ReLU pairs
-    fused on CUDA."""
+    fused on CUDA, and nn.Linear weight gradients from librank."""
     from .din import Dice
     n, i = len(layers), 0
     max_b = None
@@ -151,6 +193,12 @@ def run_tower(layers, x):
                 x = _BnAct.apply(x, layer.weight, layer.bias, layer, _activation_slope(layers[i + 1]))
                 i += 2
                 continue
+        if (FUSED and type(layer) is nn.Linear and x.is_cuda and x.dim() == 2 and x.dtype == torch.float32
+                and layer.weight.dtype == torch.float32 and MIN_BATCH <= x.shape[0]
+                and layer.out_features >= LINEAR_MIN_OUT):
+            x = _Linear.apply(x, layer.weight, layer.bias)
+            i += 1
+            continue
         x = layer(x)
         i += 1
     return x

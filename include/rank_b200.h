@@ -290,6 +290,15 @@ int rk_bn_act_bwd(const float* x, const float* g_z, int64_t B, int units, const 
                   const float* beta, float slope, const float* stats, float* g_x, float* g_gamma,
                   float* g_beta, rk_stream_t stream);
 
+/* Weight and bias gradients of a tower nn.Linear (y = x W^T + b): dW[N, K] = G^T X and db[N] = sum_b G[b, :],
+ * fp32 FMA.  Row b of x[B, K] starts at x + b*ldx, of g[B, N] at g + b*ldg (ldx >= K, ldg >= N); db may be
+ * NULL (no bias).  The batch is split into slabs whose partial sums a second launch adds in a fixed order:
+ * partials holds rk_linear_wgrad_scratch_floats(B, K, N) floats (0: may be NULL).  Bit-identical from run to
+ * run; no allocation, no synchronisation. */
+int64_t rk_linear_wgrad_scratch_floats(int64_t B, int K, int N);   /* -1 for B, K or N < 1 */
+int rk_linear_wgrad(const float* x, int64_t ldx, const float* g, int64_t ldg, int64_t B, int K, int N,
+                    float* dW, float* db, float* partials, rk_stream_t stream);
+
 /* ---- row-wise Adam on the touched rows of a table (SURVEY 8(f) item 3; opt-in: the reference
  *      uses dense optim.Adam, e.g. DeepFM/deepfm.py:226) ---------------------------------------
  * rows[n]: distinct row numbers, grads[n, D]: their summed gradient rows (a coalesced sparse
