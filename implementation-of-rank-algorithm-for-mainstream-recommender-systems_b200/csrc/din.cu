@@ -1,17 +1,27 @@
 // din.cu — DIN hot path: every gather of DIN.forward (DIN/din.py:294-305), the local activation
 // unit din_attention (DIN/din.py:42-84), the concat (:310) and the per-sample L2 norm of the
-// mini-batch-aware regulariser (:318-322), forward and backward, fp32 SIMT.
+// mini-batch-aware regulariser (:318-322), forward and backward.  fp32 SIMT at any history width
+// T >= 0; the tensor-core activation unit further down takes T <= 128.
 //
 // One CTA owns kSamples consecutive samples.  Only history positions t < len feed the
 // activation-unit MLP (padded positions get weight 0 in raw mode and exp(-2^32/sqrt(D)) = 0 in
-// softmax mode, so their scores are never observable); whole samples are packed into tiles of at
-// most kRows (b,t) rows.  Per tile:
+// softmax mode, so their scores are never observable).  The CTA's live (b,t) rows are cut into
+// tiles of at most kRows rows in sample order: whole samples while they fit (a sample with
+// len <= kRows is never split, so short samples pack several to a tile), and a sample with
+// len > kRows is cut at the tile edge and continues in the next tile.  Segment j of a tile = the
+// rows of sample s_begin + j it holds.  Per tile:
 //   gather   K rows (64 B each at D=16) -> shared memory, feature-major, with q, q-k, q*k
 //   MLP      [rows,4D]x[4D,64] -> ReLU -> [rows,64]x[64,32] -> ReLU -> .w3   (tile_gemm.cuh)
-//   pooling  masked raw / scaled-softmax weights, sum_t w_t k_t  (warp per sample, shuffles)
+//   pooling  one warp per segment:
+//     raw      the pooled vector sum_t s_t k_t is accumulated segment after segment (fixed order)
+//     softmax  online: per sample a running max m and sum S of exp(z - m); a segment with max m'
+//              rescales (S, pooled) by exp(m - max(m, m')).  att_w holds the scaled scores z_t until
+//              the sample's last segment, which rewrites them as exp(z_t - m) / S.
 // The backward never needs dW of the unit (its weights are drawn per call and unregistered,
 // DIN/din.py:61-67), so the forward keeps only the two ReLU masks as bits (12 B per row) and the
-// weights w_t; the backward is g_score -> 32 -> 64 -> 4D through the transposed weights.
+// weights w_t; the backward is g_score -> 32 -> 64 -> 4D through the transposed weights.  Its
+// softmax term sum_u w_u (g_att . k_u) = g_att . pooled, and pooled is saved in concat_all, so
+// every row's score gradient is local; g_q is summed segment after segment.
 #include <string.h>
 #include "common.cuh"
 #include <cuda_bf16.h>
@@ -65,7 +75,11 @@ struct DinSmem {
     float *score, *gw;             // [kRows]
     float *q, *gatt, *gq;          // [kSamples][D]
     int   *row_s, *row_t;          // row -> (local sample, t)
-    int   *len, *start;            // per sample: clipped length, first row in the tile list
+    int   *len;                    // [kSamples] clipped length
+    float *run_max, *run_sum;      // [kSamples] softmax running max / sum (backward: run_sum = g_att . pooled)
+    int   *seg_r0, *seg_t0;        // [kSamples + 1], [kSamples]: segment j = rows [seg_r0[j], seg_r0[j+1]),
+                                   // positions seg_t0[j] + (row - seg_r0[j]) of sample s_begin + j
+    int   *cursor;                 // [4] n_segments, n_rows, next sample, next position
     uint32_t* mask;                // [3][kRows] (backward)
     __device__ DinSmem(float* base, int D) {
         const int K1 = 4 * D;
@@ -84,14 +98,18 @@ struct DinSmem {
         row_s = (int*)p;  p += kRows;
         row_t = (int*)p;  p += kRows;
         len = (int*)p;    p += kSamples;
-        start = (int*)p;  p += kSamples + 4;
+        run_max = p;      p += kSamples;
+        run_sum = p;      p += kSamples;
+        seg_r0 = (int*)p; p += kSamples + 1;
+        seg_t0 = (int*)p; p += kSamples;
+        cursor = (int*)p; p += 4;
         mask = (uint32_t*)p;  p += 3 * kRows;
     }
     static size_t bytes(int D) {
         const int K1 = 4 * D;
         return sizeof(float) * (size_t)(K1 * kH1 + kH1 * kH2 + 2 * kH1 + 2 * kH2 + 4 + K1 * kRows +
                                         kH1 * kRows + kH2 * kRows + 2 * kRows + 3 * kSamples * D +
-                                        2 * kRows + 2 * kSamples + 4 + 3 * kRows);
+                                        2 * kRows + 4 * kSamples + 1 + kSamples + 4 + 3 * kRows);
     }
 };
 
@@ -135,455 +153,38 @@ __device__ __forceinline__ void stage_rows(const DinParams& p, const DinSmem& sm
     }
 }
 
-// Pack whole samples [s_begin, s_end) of the CTA into one tile of <= kRows rows (thread 0 plans).
-__device__ __forceinline__ int plan_tile(const DinSmem& sm, int n_samples, int s_begin, int* s_end_out) {
-    // every thread computes the same small scan: no divergence, no extra barrier
-    int rows = 0, s = s_begin;
-    while (s < n_samples && rows + sm.len[s] <= kRows) {
-        rows += sm.len[s];
-        ++s;
-    }
-    *s_end_out = s;
-    return rows;
-}
-
-__global__ void __launch_bounds__(kDinThreads)
-din_fwd_kernel(const __grid_constant__ DinParams p, float* __restrict__ concat_all,
-               float* __restrict__ norm_out, float* __restrict__ att_w, uint32_t* __restrict__ masks,
-               int32_t* err_flag) {
-    extern __shared__ __align__(16) float smem_raw[];
-    const int D = p.D, K1 = 4 * D, T = p.T;
-    DinSmem sm(smem_raw, D);
-    const MlpLayout L(D);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int64_t b0 = (int64_t)blockIdx.x * kSamples;
-    const int n_samples = (int)((p.B - b0) < kSamples ? (p.B - b0) : kSamples);
-
-    // ---- stage the per-call weights and the CTA's q rows / lengths
-    for (int i = tid; i < K1 * kH1; i += kDinThreads) sm.wA[i] = __ldg(p.mlp + L.w1t + i);
-    for (int i = tid; i < kH1 * kH2; i += kDinThreads) sm.wB[i] = __ldg(p.mlp + L.w2t + i);
-    for (int i = tid; i < kH1; i += kDinThreads) sm.vec[i] = __ldg(p.mlp + L.b1 + i);
-    for (int i = tid; i < kH2; i += kDinThreads) {
-        sm.vec[kH1 + i]       = __ldg(p.mlp + L.b2 + i);
-        sm.vec[kH1 + kH2 + i] = __ldg(p.mlp + L.w3 + i);
-    }
-    if (tid == 0) sm.vec[kH1 + 2 * kH2] = __ldg(p.mlp + L.b3);
-    for (int i = tid; i < n_samples * D; i += kDinThreads) {
-        const int s = i / D, e = i - s * D;
-        const int64_t row = checked_row(__ldg(p.tgt_idx + b0 + s), p.tgt_rows, err_flag);
-        sm.q[i] = __ldg(p.tgt_w + row * D + e);
-    }
-    if (tid < kSamples) sm.len[tid] = tid < n_samples ? clip_len(__ldg(p.his_len + b0 + tid), T) : 0;
-    __syncthreads();
-    const float* b1 = sm.vec;
-    const float* b2 = sm.vec + kH1;
-    const float* w3 = sm.vec + kH1 + kH2;
-    const float  b3 = sm.vec[kH1 + 2 * kH2];
-    const float  inv_sqrt_d = 1.0f / sqrtf((float)D);
-
-    int s_begin = 0;
-    while (s_begin < n_samples) {
-        int s_end;
-        const int n_rows = plan_tile(sm, n_samples, s_begin, &s_end);
-        // row map: tile row -> (sample, t)
-        if (tid < kSamples + 1) {
-            int acc = 0;
-            for (int s = s_begin; s < s_begin + tid && s < s_end; ++s) acc += sm.len[s];
-            sm.start[tid] = acc;     // start[j] = first row of sample s_begin + j
-        }
-        __syncthreads();
-        for (int m = tid; m < kRows; m += kDinThreads) {
-            int s = s_begin;
-            while (s + 1 < s_end && m >= sm.start[s + 1 - s_begin]) ++s;
-            sm.row_s[m] = s;
-            sm.row_t[m] = m - sm.start[s - s_begin];
-        }
-        __syncthreads();
-        if (n_rows > 0) {
-            stage_rows<true>(p, sm, b0, n_rows, err_flag);
-            __syncthreads();
-            const int m_used = (n_rows + 3) / 4 * 4;
-            // layer 1: [rows,4D] x [4D,64] + b1, ReLU
-            tile_gemm_rows<8>(sm.x, sm.wA, K1, kH1, m_used, [&](int m0, int n0, float (&acc)[4][8]) {
-#pragma unroll
-                for (int j = 0; j < 8; ++j)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) acc[i][j] = fmaxf(acc[i][j] + b1[n0 + j], 0.f);
-                store_tile_kmajor<8>(sm.h1, kRows, m0, n0, acc);
-            });
-            __syncthreads();
-            // layer 2: [rows,64] x [64,32] + b2, ReLU
-            tile_gemm_rows<4>(sm.h1, sm.wB, kH1, kH2, m_used, [&](int m0, int n0, float (&acc)[4][4]) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) acc[i][j] = fmaxf(acc[i][j] + b2[n0 + j], 0.f);
-                store_tile_kmajor<4>(sm.h2, kRows, m0, n0, acc);
-            });
-            __syncthreads();
-            // layer 3 (32 -> 1) and the two ReLU masks as bits
-            if (tid < n_rows) {
-                const int m = tid;
-                float sc = b3;
-                uint32_t m2 = 0, m1a = 0, m1b = 0;
-#pragma unroll 8
-                for (int n = 0; n < kH2; ++n) {
-                    const float h = sm.h2[n * kRows + m];
-                    sc = fmaf(h, w3[n], sc);
-                    m2 |= (h > 0.f ? 1u : 0u) << n;
-                }
-#pragma unroll 8
-                for (int n = 0; n < 32; ++n) {
-                    m1a |= (sm.h1[n * kRows + m] > 0.f ? 1u : 0u) << n;
-                    m1b |= (sm.h1[(32 + n) * kRows + m] > 0.f ? 1u : 0u) << n;
-                }
-                sm.score[m] = sc;
-                if (masks) {
-                    uint32_t* mk = masks + ((b0 + sm.row_s[m]) * T + sm.row_t[m]) * 3;
-                    mk[0] = m1a; mk[1] = m1b; mk[2] = m2;
-                }
-            }
-            __syncthreads();
-        }
-        // ---- pooling: one warp per sample of the tile
-        for (int s = s_begin + warp; s < s_end; s += kDinThreads / 32) {
-            const int len = sm.len[s], r0 = sm.start[s - s_begin];
-            float* wrow = att_w + (b0 + s) * T;
-            float* out  = concat_all + (b0 + s) * p.width + p.att_off;
-            if (len == 0) {
-                if (!p.use_softmax) {
-                    for (int t = lane; t < T; t += 32) wrow[t] = 0.f;
-                    for (int e = lane; e < D; e += 32) { out[e] = 0.f; sm.gatt[s * D + e] = 0.f; }
-                } else {  // uniform 1/T over ALL positions (they all hold the padding score)
-                    const float u = 1.0f / (float)T;
-                    for (int t = lane; t < T; t += 32) wrow[t] = u;
-                    for (int e = 0; e < D; ++e) {
-                        float a = 0.f;
-                        for (int t = lane; t < T; t += 32) {
-                            const int64_t row = checked_row(__ldg(p.his_idx + (b0 + s) * T + t), p.his_rows, err_flag);
-                            a = fmaf(u, __ldg(p.his_w + row * D + e), a);
-                        }
-                        a = warp_sum(a);
-                        if (lane == 0) { out[e] = a; sm.gatt[s * D + e] = a; }
-                    }
-                }
-                continue;
-            }
-            float inv_sum = 1.f, mx = 0.f;
-            if (p.use_softmax) {
-                mx = -INFINITY;
-                for (int t = lane; t < len; t += 32) mx = fmaxf(mx, sm.score[r0 + t] * inv_sqrt_d);
-                mx = warp_max(mx);
-                float sum = 0.f;
-                for (int t = lane; t < len; t += 32) sum += expf(sm.score[r0 + t] * inv_sqrt_d - mx);
-                inv_sum = 1.0f / warp_sum(sum);
-            }
-            for (int t = lane; t < T; t += 32) {
-                float w = 0.f;
-                if (t < len) {
-                    w = p.use_softmax ? expf(sm.score[r0 + t] * inv_sqrt_d - mx) * inv_sum : sm.score[r0 + t];
-                    sm.gw[r0 + t] = w;
-                }
-                wrow[t] = w;
-            }
-            __syncwarp();
-            for (int e = 0; e < D; ++e) {
-                float a = 0.f;
-                for (int t = lane; t < len; t += 32) a = fmaf(sm.gw[r0 + t], sm.x[(D + e) * kRows + r0 + t], a);
-                a = warp_sum(a);
-                if (lane == 0) { out[e] = a; sm.gatt[s * D + e] = a; }
-            }
-        }
-        __syncthreads();
-        s_begin = s_end;
-    }
-
-    // ---- assemble the rest of the concat row and the L2 norm: one warp per sample
-    for (int s = warp; s < n_samples; s += kDinThreads / 32) {
-        const int64_t b = b0 + s;
-        float* out = concat_all + b * p.width;
-        float ss = 0.f;
-        for (int c = lane; c < p.width; c += 32) {
-            float v;
-            if (c < p.n_dense) {
-                v = __ldg(p.dense_col[c] + b * p.dense_stride);
-                out[c] = v;
-            } else if (c >= p.att_off && c < p.att_off + D) {
-                v = sm.gatt[s * D + c - p.att_off];        // pooled above (kept in shared memory)
-            } else if (c >= p.tgt_off && c < p.tgt_off + D) {
-                v = sm.q[s * D + c - p.tgt_off];
-                out[c] = v;
-            } else {
-                v = 0.f;
-                for (int f = 0; f < p.cat.F; ++f)
-                    if (c >= p.cat.off[f] && c < p.cat.off[f] + p.cat.dim[f]) {
-                        const int64_t row = checked_row(__ldg(p.cat.idx[f] + b), p.cat.rows[f], err_flag);
-                        v = __ldg(p.cat.weight[f] + row * p.cat.dim[f] + c - p.cat.off[f]);
-                    }
-                out[c] = v;
-            }
-            if (c >= p.l2_from) ss = fmaf(v, v, ss);
-        }
-        ss = warp_sum(ss);
-        if (lane == 0 && norm_out) norm_out[b] = sqrtf(ss);
-    }
-}
-
-// Backward.  g_row[B,width]: gradient w.r.t. every column of the concat row INCLUDING what flows
-// back through the attention into q (target columns) — these are the per-occurrence gradients of
-// the category / target tables.  g_hist[B,T,D]: per-occurrence gradients of the history table
-// (written for live positions only).
-__global__ void __launch_bounds__(kDinThreads)
-din_bwd_kernel(const __grid_constant__ DinParams p, const float* __restrict__ concat_all,
-               const float* __restrict__ norm, const float* __restrict__ att_w,
-               const uint32_t* __restrict__ masks, const float* __restrict__ g_concat,
-               const float* __restrict__ g_norm, float* __restrict__ g_row,
-               float* __restrict__ g_hist, int32_t* err_flag) {
-    extern __shared__ __align__(16) float smem_raw[];
-    const int D = p.D, K1 = 4 * D, T = p.T;
-    DinSmem sm(smem_raw, D);
-    const MlpLayout L(D);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int64_t b0 = (int64_t)blockIdx.x * kSamples;
-    const int n_samples = (int)((p.B - b0) < kSamples ? (p.B - b0) : kSamples);
-
-    // weights in their registered orientation: B operands of the transposed products
-    for (int i = tid; i < kH1 * K1; i += kDinThreads) sm.wA[i] = __ldg(p.mlp + L.w1 + i);   // [64][K1]
-    for (int i = tid; i < kH2 * kH1; i += kDinThreads) sm.wB[i] = __ldg(p.mlp + L.w2 + i);  // [32][64]
-    for (int i = tid; i < kH2; i += kDinThreads) sm.vec[i] = __ldg(p.mlp + L.w3 + i);
-    if (tid < kSamples) sm.len[tid] = tid < n_samples ? clip_len(__ldg(p.his_len + b0 + tid), T) : 0;
-    // per sample: q, and g_att = upstream gradient of the attention output (tower + L2 term)
-    for (int i = tid; i < n_samples * D; i += kDinThreads) {
-        const int s = i / D, e = i - s * D;
-        const int64_t b = b0 + s;
-        sm.q[i] = concat_all[b * p.width + p.tgt_off + e];
-        float g = g_concat ? g_concat[b * p.width + p.att_off + e] : 0.f;
-        if (g_norm) {
-            const float nv = norm[b];
-            if (nv > 0.f) g = fmaf(g_norm[b] / nv, concat_all[b * p.width + p.att_off + e], g);
-        }
-        sm.gatt[i] = g;
-        sm.gq[i]   = 0.f;
-    }
-    __syncthreads();
-    const float* w3 = sm.vec;
-    const float  inv_sqrt_d = 1.0f / sqrtf((float)D);
-
-    int s_begin = 0;
-    while (s_begin < n_samples) {
-        int s_end;
-        const int n_rows = plan_tile(sm, n_samples, s_begin, &s_end);
-        if (tid < kSamples + 1) {
-            int acc = 0;
-            for (int s = s_begin; s < s_begin + tid && s < s_end; ++s) acc += sm.len[s];
-            sm.start[tid] = acc;
-        }
-        __syncthreads();
-        for (int m = tid; m < kRows; m += kDinThreads) {
-            int s = s_begin;
-            while (s + 1 < s_end && m >= sm.start[s + 1 - s_begin]) ++s;
-            sm.row_s[m] = s;
-            sm.row_t[m] = m - sm.start[s - s_begin];
-        }
-        __syncthreads();
-        if (n_rows > 0) {
-            stage_rows<false>(p, sm, b0, n_rows, err_flag);      // K rows -> x[D..2D)
-            __syncthreads();
-            // g_w[row] = g_att . k_row ; load w_t and the ReLU masks
-            if (tid < kRows) {
-                const int m = tid;
-                float gw = 0.f, w = 0.f;
-                uint32_t k0 = 0, k1 = 0, k2 = 0;
-                if (m < n_rows) {
-                    const int s = sm.row_s[m], t = sm.row_t[m];
-                    for (int e = 0; e < D; ++e) gw = fmaf(sm.gatt[s * D + e], sm.x[(D + e) * kRows + m], gw);
-                    w = att_w[(b0 + s) * T + t];
-                    const uint32_t* mk = masks + ((b0 + s) * T + t) * 3;
-                    k0 = mk[0]; k1 = mk[1]; k2 = mk[2];
-                }
-                sm.gw[m] = gw;
-                sm.score[m] = w;
-                sm.mask[m] = k0; sm.mask[kRows + m] = k1; sm.mask[2 * kRows + m] = k2;
-            }
-            __syncthreads();
-            // softmax backward needs sum_u w_u g_w_u per sample (warp per sample)
-            if (p.use_softmax) {
-                for (int s = s_begin + warp; s < s_end; s += kDinThreads / 32) {
-                    const int len = sm.len[s], r0 = sm.start[s - s_begin];
-                    float dot = 0.f;
-                    for (int t = lane; t < len; t += 32) dot = fmaf(sm.score[r0 + t], sm.gw[r0 + t], dot);
-                    dot = warp_sum(dot);
-                    for (int t = lane; t < len; t += 32)
-                        sm.gw[r0 + t] = sm.score[r0 + t] * (sm.gw[r0 + t] - dot) * inv_sqrt_d;
-                }
-                __syncthreads();
-            }
-            // g_z2[n][m] = g_s[m] * w3[n] * relu2'  -> h2 region
-            if (tid < kRows) {
-                const int m = tid;
-                const float gs = m < n_rows ? sm.gw[m] : 0.f;
-                const uint32_t k2 = sm.mask[2 * kRows + m];
-#pragma unroll 8
-                for (int n = 0; n < kH2; ++n) sm.h2[n * kRows + m] = ((k2 >> n) & 1u) ? gs * w3[n] : 0.f;
-            }
-            __syncthreads();
-            const int m_used = (n_rows + 3) / 4 * 4;
-            // g_z1 = (g_z2 x W2) * relu1'   [rows,32]x[32,64]
-            tile_gemm_rows<8>(sm.h2, sm.wB, kH2, kH1, m_used, [&](int m0, int n0, float (&acc)[4][8]) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const uint32_t bits = sm.mask[(n0 >> 5) * kRows + m0 + i] >> (n0 & 31);
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) acc[i][j] = ((bits >> j) & 1u) ? acc[i][j] : 0.f;
-                }
-                store_tile_kmajor<8>(sm.h1, kRows, m0, n0, acc);
-            });
-            __syncthreads();
-            // g_cross = g_z1 x W1   [rows,64]x[64,4D]  -> reuse x[0..D) and x[2D..4D) ... keep K rows:
-            // write g_cross into a scratch that does not overlap x[D..2D): use h-major temp in h1? no:
-            // h1 is this product's A operand.  g_cross goes to x rows {0..D) U [2D,4D) directly and its
-            // k-block [D,2D) into h2 (free now, D <= 32 rows).
-            tile_gemm_rows<4>(sm.h1, sm.wA, kH1, K1, m_used, [&](int m0, int n0, float (&acc)[4][4]) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int c = n0 + j;
-                    float* dst = (c >= D && c < 2 * D) ? sm.h2 + (c - D) * kRows : sm.x + c * kRows;
-                    *reinterpret_cast<float4*>(dst + m0) = make_float4(acc[0][j], acc[1][j], acc[2][j], acc[3][j]);
-                }
-            });
-            __syncthreads();
-            // per row: g_k = w_t g_att + gc_k - gc_d + gc_p * q ; g_q_row = gc_q + gc_d + gc_p * k
-            for (int item = tid; item < D * kRows; item += kDinThreads) {
-                const int e = item / kRows, m = item - e * kRows;
-                if (m < n_rows) {
-                    const int s = sm.row_s[m], t = sm.row_t[m];
-                    const float k  = sm.x[(D + e) * kRows + m];
-                    const float q  = sm.q[s * D + e];
-                    const float gq = sm.x[e * kRows + m];
-                    const float gk = sm.h2[e * kRows + m];
-                    const float gd = sm.x[(2 * D + e) * kRows + m];
-                    const float gp = sm.x[(3 * D + e) * kRows + m];
-                    const float w  = sm.score[m];
-                    // overwrite x[e] with this row's contribution to g_q; the K row with g_k
-                    sm.x[e * kRows + m]       = gq + gd + gp * k;
-                    sm.x[(D + e) * kRows + m] = fmaf(w, sm.gatt[s * D + e], gk - gd + gp * q);
-                    (void)t;
-                }
-            }
-            __syncthreads();
-            // write g_k rows (coalesced over e inside a row) and reduce g_q over each sample's rows
-            for (int item = tid; item < (D / 4) * kRows; item += kDinThreads) {
-                const int c4 = item / kRows, m = item - c4 * kRows;
-                if (m < n_rows) {
-                    const float* src = sm.x + (D + 4 * c4) * kRows + m;
-                    *reinterpret_cast<float4*>(g_hist + ((b0 + sm.row_s[m]) * T + sm.row_t[m]) * D + 4 * c4) =
-                        make_float4(src[0], src[kRows], src[2 * kRows], src[3 * kRows]);
-                }
-            }
-            for (int s = s_begin + warp; s < s_end; s += kDinThreads / 32) {
-                const int len = sm.len[s], r0 = sm.start[s - s_begin];
-                for (int e = 0; e < D; ++e) {
-                    float a = 0.f;
-                    for (int t = lane; t < len; t += 32) a += sm.x[e * kRows + r0 + t];
-                    a = warp_sum(a);
-                    if (lane == 0) sm.gq[s * D + e] = a;
-                }
-            }
-            __syncthreads();
-        }
-        // samples with no history in softmax mode: uniform weights, gradient g_att / T everywhere
-        if (p.use_softmax) {
-            for (int s = s_begin; s < s_end; ++s) {
-                if (sm.len[s] != 0) continue;
-                const float u = 1.0f / (float)T;
-                for (int i = tid; i < T * D; i += kDinThreads)
-                    g_hist[(b0 + s) * T * D + i] = u * sm.gatt[s * D + (i % D)];
-            }
-        }
-        __syncthreads();
-        s_begin = s_end;
-    }
-
-    // ---- gradient of the concat row: tower gradient + L2 term (+ attention's d/dq on the target)
-    for (int s = warp; s < n_samples; s += kDinThreads / 32) {
-        const int64_t b = b0 + s;
-        float scale = 0.f;
-        if (g_norm) {
-            const float nv = norm[b];
-            scale = nv > 0.f ? g_norm[b] / nv : 0.f;
-        }
-        for (int c = lane; c < p.width; c += 32) {
-            float g = g_concat ? g_concat[b * p.width + c] : 0.f;
-            if (c >= p.l2_from) g = fmaf(scale, concat_all[b * p.width + c], g);
-            if (c >= p.tgt_off && c < p.tgt_off + D) g += sm.gq[s * D + c - p.tgt_off];
-            g_row[b * p.width + c] = g;
-        }
-    }
-}
-
-// ===========================================================================================
-// Histories wider than one tile (T > kRows), fp32 SIMT.  Same CTA shape, same gather, same MLP
-// and the same per-row backward as the kernels above; what changes is the tile planner and the
-// pooling.  A tile is cut from the CTA's live rows in sample order: whole samples while they fit
-// (a sample with len <= kRows is never split, so short samples pack several to a tile exactly as
-// plan_tile packs them), and a sample with len > kRows is cut at the tile edge and continues in the
-// next tile.  Segment j of a tile = the rows of sample s_begin + j it holds.
-//   raw      the pooled vector sum_t s_t k_t is accumulated segment after segment (fixed order)
-//   softmax  online: per sample a running max m and sum S of exp(z - m); a segment with max m'
-//            rescales (S, pooled) by exp(m - max(m, m')).  att_w holds the scaled scores z_t until
-//            the sample's last segment, which rewrites them as exp(z_t - m) / S.
-// Backward: the softmax term sum_u w_u (g_att . k_u) = g_att . pooled, and pooled is saved in
-// concat_all, so every row's score gradient is local; g_q is summed segment after segment.
-// ===========================================================================================
-struct DinLongSmem {
-    float *run_max, *run_sum;   // [kSamples] softmax running max / sum (backward: run_sum = g_att . pooled)
-    int   *seg_r0, *seg_t0;     // [kSamples + 1], [kSamples]: segment j = rows [seg_r0[j], seg_r0[j+1]),
-                                // positions seg_t0[j] + (row - seg_r0[j]) of sample s_begin + j
-    int   *cursor;              // [4] n_segments, n_rows, next sample, next position
-    __device__ DinLongSmem(float* base) {
-        float* p = base;
-        run_max = p;  p += kSamples;
-        run_sum = p;  p += kSamples;
-        seg_r0 = (int*)p;  p += kSamples + 1;
-        seg_t0 = (int*)p;  p += kSamples;
-        cursor = (int*)p;
-    }
-    static constexpr size_t kBytes = sizeof(float) * (4 * kSamples + 1 + 4);
-};
-
 // Thread 0 plans the tile that starts at position t_begin of sample s_begin (tests/test_din_long.py
 // restates this planner).
-__device__ __forceinline__ void plan_long_tile(const DinSmem& sm, const DinLongSmem& ls, int n_samples,
-                                               int s_begin, int t_begin) {
+__device__ __forceinline__ void plan_tile(const DinSmem& sm, int n_samples, int s_begin, int t_begin) {
     int rows = 0, j = 0, s = s_begin, t0 = t_begin;
     while (s < n_samples) {
         const int rem = sm.len[s] - t0;
         if (rem <= kRows - rows) {                      // the rest of the sample fits
-            ls.seg_r0[j] = rows;  ls.seg_t0[j] = t0;  ++j;
+            sm.seg_r0[j] = rows;  sm.seg_t0[j] = t0;  ++j;
             rows += rem;  ++s;  t0 = 0;
             continue;
         }
         if (sm.len[s] <= kRows || rows == kRows) break;  // a short sample is never split
-        ls.seg_r0[j] = rows;  ls.seg_t0[j] = t0;  ++j;   // a long one fills the tile
+        sm.seg_r0[j] = rows;  sm.seg_t0[j] = t0;  ++j;   // a long one fills the tile
         t0 += kRows - rows;  rows = kRows;
         break;
     }
-    ls.seg_r0[j] = rows;
-    ls.cursor[0] = j;  ls.cursor[1] = rows;  ls.cursor[2] = s;  ls.cursor[3] = t0;
+    sm.seg_r0[j] = rows;
+    sm.cursor[0] = j;  sm.cursor[1] = rows;  sm.cursor[2] = s;  sm.cursor[3] = t0;
 }
 
-__device__ __forceinline__ void long_row_map(const DinSmem& sm, const DinLongSmem& ls, int n_seg, int s_begin) {
+__device__ __forceinline__ void row_map(const DinSmem& sm, int n_seg, int s_begin) {
     for (int m = threadIdx.x; m < kRows; m += kDinThreads) {
         int j = 0;
-        while (j + 1 < n_seg && m >= ls.seg_r0[j + 1]) ++j;
+        while (j + 1 < n_seg && m >= sm.seg_r0[j + 1]) ++j;
         sm.row_s[m] = s_begin + j;
-        sm.row_t[m] = ls.seg_t0[j] + m - ls.seg_r0[j];
+        sm.row_t[m] = sm.seg_t0[j] + m - sm.seg_r0[j];
     }
 }
 
-// din_fwd_kernel's activation unit on one staged tile: layers 1-3, scores -> sm.score, mask bits -> masks.
-__device__ __forceinline__ void long_mlp_fwd(const DinParams& p, const DinSmem& sm, int64_t b0, int n_rows,
-                                             uint32_t* masks) {
+// The activation unit on one staged tile: layers 1-3, scores -> sm.score, mask bits -> masks.
+__device__ __forceinline__ void mlp_fwd(const DinParams& p, const DinSmem& sm, int64_t b0, int n_rows,
+                                        uint32_t* masks) {
     const int K1 = 4 * p.D, tid = threadIdx.x;
     const float* b1 = sm.vec;
     const float* b2 = sm.vec + kH1;
@@ -630,10 +231,14 @@ __device__ __forceinline__ void long_mlp_fwd(const DinParams& p, const DinSmem& 
     __syncthreads();
 }
 
-// Softmax mode, len == 0: every position holds the padding score, so the weights are 1/T over all T
-// positions (the reference's quirk).  One warp; each lane sums whole rows, then the lanes reduce.
-__device__ __forceinline__ void long_pool_empty(const DinParams& p, int64_t b, float* pooled, int32_t* err_flag) {
+// Softmax mode, len == 0, T > 0: every position holds the padding score, so the weights are 1/T over
+// all T positions (the reference's quirk).  Each row is weighted by u = 1/T before it is added, as the
+// reference weights it: a batch of empty histories over the same padding row gives every sample the
+// same pooled vector, and the tower's batch norm turns any ulp by which it differs into its bias
+// gradients.  One warp; each lane sums whole rows in t order, then the lanes reduce.
+__device__ __forceinline__ void pool_empty(const DinParams& p, int64_t b, float* pooled, int32_t* err_flag) {
     const int D = p.D, D4 = D / 4, T = p.T, lane = threadIdx.x & 31;
+    const float u = 1.0f / (float)T;
     float4 a[8];
 #pragma unroll
     for (int c = 0; c < 8; ++c) a[c] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -644,22 +249,22 @@ __device__ __forceinline__ void long_pool_empty(const DinParams& p, int64_t b, f
         for (int c = 0; c < 8; ++c)
             if (c < D4) {
                 const float4 v = __ldg(k + c);
-                a[c].x += v.x; a[c].y += v.y; a[c].z += v.z; a[c].w += v.w;
+                a[c].x = fmaf(u, v.x, a[c].x); a[c].y = fmaf(u, v.y, a[c].y);
+                a[c].z = fmaf(u, v.z, a[c].z); a[c].w = fmaf(u, v.w, a[c].w);
             }
     }
-    const float u = 1.0f / (float)T;
 #pragma unroll
     for (int c = 0; c < 8; ++c)
         if (c < D4) {
             const float v[4] = {warp_sum(a[c].x), warp_sum(a[c].y), warp_sum(a[c].z), warp_sum(a[c].w)};
             if (lane == 0)
-                for (int e = 0; e < 4; ++e) pooled[4 * c + e] = u * v[e];
+                for (int e = 0; e < 4; ++e) pooled[4 * c + e] = v[e];
         }
 }
 
-// din_fwd_kernel's last step: the rest of the concat row and the L2 norm, one warp per sample.
-__device__ __forceinline__ void long_concat_norm(const DinParams& p, const DinSmem& sm, int64_t b0, int n_samples,
-                                                 float* concat_all, float* norm_out, int32_t* err_flag) {
+// The forward's last step: the rest of the concat row and the L2 norm, one warp per sample.
+__device__ __forceinline__ void concat_norm(const DinParams& p, const DinSmem& sm, int64_t b0, int n_samples,
+                                            float* concat_all, float* norm_out, int32_t* err_flag) {
     const int D = p.D, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int s = warp; s < n_samples; s += kDinThreads / 32) {
         const int64_t b = b0 + s;
@@ -671,7 +276,7 @@ __device__ __forceinline__ void long_concat_norm(const DinParams& p, const DinSm
                 v = __ldg(p.dense_col[c] + b * p.dense_stride);
                 out[c] = v;
             } else if (c >= p.att_off && c < p.att_off + D) {
-                v = sm.gatt[s * D + c - p.att_off];
+                v = sm.gatt[s * D + c - p.att_off];        // pooled (kept in shared memory)
             } else if (c >= p.tgt_off && c < p.tgt_off + D) {
                 v = sm.q[s * D + c - p.tgt_off];
                 out[c] = v;
@@ -691,19 +296,22 @@ __device__ __forceinline__ void long_concat_norm(const DinParams& p, const DinSm
     }
 }
 
-__global__ void __launch_bounds__(kDinThreads)
-din_fwd_long_kernel(const __grid_constant__ DinParams p, float* __restrict__ concat_all,
-                    float* __restrict__ norm_out, float* __restrict__ att_w, uint32_t* __restrict__ masks,
-                    int32_t* err_flag) {
+// Shared memory holds this kernel at 2 CTAs per SM, so it may use up to 128 registers at no cost in
+// occupancy; with that bound stated ptxas schedules it at ~100 registers, which measured 0.4-2.4 % faster
+// (hot path, T = 1..256) than the ~75 it picks unbounded.
+__global__ void __launch_bounds__(kDinThreads, 2)
+din_fwd_kernel(const __grid_constant__ DinParams p, float* __restrict__ concat_all,
+               float* __restrict__ norm_out, float* __restrict__ att_w, uint32_t* __restrict__ masks,
+               int32_t* err_flag) {
     extern __shared__ __align__(16) float smem_raw[];
     const int D = p.D, K1 = 4 * D, T = p.T;
     DinSmem sm(smem_raw, D);
-    DinLongSmem ls(reinterpret_cast<float*>(sm.mask + 3 * kRows));   // right after the DinSmem carve-up
     const MlpLayout L(D);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t b0 = (int64_t)blockIdx.x * kSamples;
     const int n_samples = (int)((p.B - b0) < kSamples ? (p.B - b0) : kSamples);
 
+    // ---- stage the per-call weights and the CTA's q rows / lengths
     for (int i = tid; i < K1 * kH1; i += kDinThreads) sm.wA[i] = __ldg(p.mlp + L.w1t + i);
     for (int i = tid; i < kH1 * kH2; i += kDinThreads) sm.wB[i] = __ldg(p.mlp + L.w2t + i);
     for (int i = tid; i < kH1; i += kDinThreads) sm.vec[i] = __ldg(p.mlp + L.b1 + i);
@@ -720,34 +328,34 @@ din_fwd_long_kernel(const __grid_constant__ DinParams p, float* __restrict__ con
     for (int i = tid; i < kSamples * D; i += kDinThreads) sm.gatt[i] = 0.f;   // pooled, accumulated per segment
     if (tid < kSamples) {
         sm.len[tid] = tid < n_samples ? clip_len(__ldg(p.his_len + b0 + tid), T) : 0;
-        ls.run_max[tid] = -INFINITY;
-        ls.run_sum[tid] = 0.f;
+        sm.run_max[tid] = -INFINITY;
+        sm.run_sum[tid] = 0.f;
     }
     __syncthreads();
     const float inv_sqrt_d = 1.0f / sqrtf((float)D);
 
     int s_begin = 0, t_begin = 0;
     while (s_begin < n_samples) {
-        if (tid == 0) plan_long_tile(sm, ls, n_samples, s_begin, t_begin);
+        if (tid == 0) plan_tile(sm, n_samples, s_begin, t_begin);
         __syncthreads();
-        const int n_seg = ls.cursor[0], n_rows = ls.cursor[1], s_next = ls.cursor[2], t_next = ls.cursor[3];
-        long_row_map(sm, ls, n_seg, s_begin);
+        const int n_seg = sm.cursor[0], n_rows = sm.cursor[1], s_next = sm.cursor[2], t_next = sm.cursor[3];
+        row_map(sm, n_seg, s_begin);
         __syncthreads();
         if (n_rows > 0) {
             stage_rows<true>(p, sm, b0, n_rows, err_flag);
             __syncthreads();
-            long_mlp_fwd(p, sm, b0, n_rows, masks);
+            mlp_fwd(p, sm, b0, n_rows, masks);
         }
         // ---- pooling: one warp per segment
         for (int j = warp; j < n_seg; j += kDinThreads / 32) {
             const int s = s_begin + j, len = sm.len[s];
-            const int r0 = ls.seg_r0[j], n = ls.seg_r0[j + 1] - r0, t0 = ls.seg_t0[j];
+            const int r0 = sm.seg_r0[j], n = sm.seg_r0[j + 1] - r0, t0 = sm.seg_t0[j];
             float* wrow = att_w + (b0 + s) * T;
             float* pooled = sm.gatt + s * D;
             if (len == 0) {
-                if (p.use_softmax) {
+                if (p.use_softmax && T > 0) {          // at T == 0 there is nothing to pool: pooled stays 0
                     for (int t = lane; t < T; t += 32) wrow[t] = 1.0f / (float)T;
-                    long_pool_empty(p, b0 + s, pooled, err_flag);
+                    pool_empty(p, b0 + s, pooled, err_flag);
                 } else {
                     for (int t = lane; t < T; t += 32) wrow[t] = 0.f;
                 }
@@ -756,8 +364,8 @@ din_fwd_long_kernel(const __grid_constant__ DinParams p, float* __restrict__ con
                 if (p.use_softmax) {
                     float mx = -INFINITY;
                     for (int r = lane; r < n; r += 32) mx = fmaxf(mx, sm.score[r0 + r] * inv_sqrt_d);
-                    mx = fmaxf(warp_max(mx), ls.run_max[s]);
-                    scale = expf(ls.run_max[s] - mx);
+                    mx = fmaxf(warp_max(mx), sm.run_max[s]);
+                    scale = expf(sm.run_max[s] - mx);
                     float sum = 0.f;
                     for (int r = lane; r < n; r += 32) {
                         const float z = sm.score[r0 + r] * inv_sqrt_d, e = expf(z - mx);
@@ -767,7 +375,7 @@ din_fwd_long_kernel(const __grid_constant__ DinParams p, float* __restrict__ con
                     }
                     sum = warp_sum(sum);
                     __syncwarp();
-                    if (lane == 0) { ls.run_sum[s] = fmaf(ls.run_sum[s], scale, sum); ls.run_max[s] = mx; }
+                    if (lane == 0) { sm.run_sum[s] = fmaf(sm.run_sum[s], scale, sum); sm.run_max[s] = mx; }
                 } else {
                     for (int r = lane; r < n; r += 32) {
                         const float w = sm.score[r0 + r];
@@ -785,7 +393,7 @@ din_fwd_long_kernel(const __grid_constant__ DinParams p, float* __restrict__ con
                 if (t0 + n == len) {                       // the sample's last segment
                     __syncwarp();
                     if (p.use_softmax) {
-                        const float mx = ls.run_max[s], inv_sum = 1.0f / ls.run_sum[s];
+                        const float mx = sm.run_max[s], inv_sum = 1.0f / sm.run_sum[s];
                         for (int t = lane; t < T; t += 32) wrow[t] = t < len ? expf(wrow[t] - mx) * inv_sum : 0.f;
                         for (int e = lane; e < D; e += 32) pooled[e] *= inv_sum;
                     } else {
@@ -801,28 +409,33 @@ din_fwd_long_kernel(const __grid_constant__ DinParams p, float* __restrict__ con
         s_begin = s_next;
         t_begin = t_next;
     }
-    long_concat_norm(p, sm, b0, n_samples, concat_all, norm_out, err_flag);
+    concat_norm(p, sm, b0, n_samples, concat_all, norm_out, err_flag);
 }
 
+// Backward.  g_row[B,width]: gradient w.r.t. every column of the concat row INCLUDING what flows
+// back through the attention into q (target columns) — these are the per-occurrence gradients of
+// the category / target tables.  g_hist[B,T,D]: per-occurrence gradients of the history table
+// (written for live positions only).
 __global__ void __launch_bounds__(kDinThreads)
-din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict__ concat_all,
-                    const float* __restrict__ norm, const float* __restrict__ att_w,
-                    const uint32_t* __restrict__ masks, const float* __restrict__ g_concat,
-                    const float* __restrict__ g_norm, float* __restrict__ g_row,
-                    float* __restrict__ g_hist, int32_t* err_flag) {
+din_bwd_kernel(const __grid_constant__ DinParams p, const float* __restrict__ concat_all,
+               const float* __restrict__ norm, const float* __restrict__ att_w,
+               const uint32_t* __restrict__ masks, const float* __restrict__ g_concat,
+               const float* __restrict__ g_norm, float* __restrict__ g_row,
+               float* __restrict__ g_hist, int32_t* err_flag) {
     extern __shared__ __align__(16) float smem_raw[];
     const int D = p.D, K1 = 4 * D, T = p.T;
     DinSmem sm(smem_raw, D);
-    DinLongSmem ls(reinterpret_cast<float*>(sm.mask + 3 * kRows));   // right after the DinSmem carve-up
     const MlpLayout L(D);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t b0 = (int64_t)blockIdx.x * kSamples;
     const int n_samples = (int)((p.B - b0) < kSamples ? (p.B - b0) : kSamples);
 
+    // weights in their registered orientation: B operands of the transposed products
     for (int i = tid; i < kH1 * K1; i += kDinThreads) sm.wA[i] = __ldg(p.mlp + L.w1 + i);   // [64][K1]
     for (int i = tid; i < kH2 * kH1; i += kDinThreads) sm.wB[i] = __ldg(p.mlp + L.w2 + i);  // [32][64]
     for (int i = tid; i < kH2; i += kDinThreads) sm.vec[i] = __ldg(p.mlp + L.w3 + i);
     if (tid < kSamples) sm.len[tid] = tid < n_samples ? clip_len(__ldg(p.his_len + b0 + tid), T) : 0;
+    // per sample: q, and g_att = upstream gradient of the attention output (tower + L2 term)
     for (int i = tid; i < n_samples * D; i += kDinThreads) {
         const int s = i / D, e = i - s * D;
         const int64_t b = b0 + s;
@@ -840,7 +453,7 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
     if (tid < n_samples) {
         float dot = 0.f;
         for (int e = 0; e < D; ++e) dot = fmaf(sm.gatt[tid * D + e], concat_all[(b0 + tid) * p.width + p.att_off + e], dot);
-        ls.run_sum[tid] = dot;
+        sm.run_sum[tid] = dot;
     }
     __syncthreads();
     const float* w3 = sm.vec;
@@ -848,10 +461,10 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
 
     int s_begin = 0, t_begin = 0;
     while (s_begin < n_samples) {
-        if (tid == 0) plan_long_tile(sm, ls, n_samples, s_begin, t_begin);
+        if (tid == 0) plan_tile(sm, n_samples, s_begin, t_begin);
         __syncthreads();
-        const int n_seg = ls.cursor[0], n_rows = ls.cursor[1], s_next = ls.cursor[2], t_next = ls.cursor[3];
-        long_row_map(sm, ls, n_seg, s_begin);
+        const int n_seg = sm.cursor[0], n_rows = sm.cursor[1], s_next = sm.cursor[2], t_next = sm.cursor[3];
+        row_map(sm, n_seg, s_begin);
         __syncthreads();
         if (n_rows > 0) {
             stage_rows<false>(p, sm, b0, n_rows, err_flag);      // K rows -> x[D..2D)
@@ -866,7 +479,7 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
                     float gw = 0.f;
                     for (int e = 0; e < D; ++e) gw = fmaf(sm.gatt[s * D + e], sm.x[(D + e) * kRows + m], gw);
                     w = att_w[(b0 + s) * T + t];
-                    gs = p.use_softmax ? w * (gw - ls.run_sum[s]) * inv_sqrt_d : gw;
+                    gs = p.use_softmax ? w * (gw - sm.run_sum[s]) * inv_sqrt_d : gw;
                     const uint32_t* mk = masks + ((b0 + s) * T + t) * 3;
                     k0 = mk[0]; k1 = mk[1]; k2 = mk[2];
                 }
@@ -889,7 +502,8 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
                 store_tile_kmajor<8>(sm.h1, kRows, m0, n0, acc);
             });
             __syncthreads();
-            // g_cross = g_z1 x W1   [rows,64]x[64,4D]: k-block [D,2D) into h2, the rest over x (as din_bwd_kernel)
+            // g_cross = g_z1 x W1   [rows,64]x[64,4D]: h1 is this product's A operand, so its k-block
+            // [D,2D) goes to h2 (free now, D <= 32 rows) and the rest over x, keeping the K rows in x[D..2D)
             tile_gemm_rows<4>(sm.h1, sm.wA, kH1, K1, m_used, [&](int m0, int n0, float (&acc)[4][4]) {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
@@ -912,6 +526,7 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
                 }
             }
             __syncthreads();
+            // write g_k rows (coalesced over e inside a row)
             for (int item = tid; item < (D / 4) * kRows; item += kDinThreads) {
                 const int c4 = item / kRows, m = item - c4 * kRows;
                 if (m < n_rows) {
@@ -922,7 +537,7 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
             }
             // g_q: each segment's rows, added to the sample's sum segment after segment
             for (int j = warp; j < n_seg; j += kDinThreads / 32) {
-                const int s = s_begin + j, r0 = ls.seg_r0[j], n = ls.seg_r0[j + 1] - r0;
+                const int s = s_begin + j, r0 = sm.seg_r0[j], n = sm.seg_r0[j + 1] - r0;
                 if (n == 0) continue;
                 for (int e = 0; e < D; ++e) {
                     float a = 0.f;
@@ -947,7 +562,7 @@ din_bwd_long_kernel(const __grid_constant__ DinParams p, const float* __restrict
         t_begin = t_next;
     }
 
-    // ---- gradient of the concat row (as din_bwd_kernel)
+    // ---- gradient of the concat row: tower gradient + L2 term (+ attention's d/dq on the target)
     for (int s = warp; s < n_samples; s += kDinThreads / 32) {
         const int64_t b = b0 + s;
         float scale = 0.f;
@@ -1890,11 +1505,11 @@ din_bwd_tc_kernel(const __grid_constant__ DinParams p, const float* __restrict__
 
 }  // namespace rk
 
-// Histories wider than one tile: the DinSmem carve-up plus the segment / running-softmax state.
+// The fp32 kernels: one CTA per kSamples samples, the DinSmem carve-up as dynamic shared memory.
 template <class Kernel, class... Args>
-static int din_launch_long(Kernel kernel, int grid, int D, rk_stream_t stream, Args... args) {
+static int din_launch(Kernel kernel, int grid, int D, rk_stream_t stream, Args... args) {
     using namespace rk;
-    const size_t smem = DinSmem::bytes(D) + DinLongSmem::kBytes;
+    const size_t smem = DinSmem::bytes(D);
     RK_CHECK_ARG(smem <= 227 * 1024, "din: %zu bytes of shared memory", smem);
     RK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kernel<<<grid, kDinThreads, smem, (cudaStream_t)stream>>>(args...);
@@ -1945,14 +1560,6 @@ static int din_pack(const rk_din_args_t* a, rk::DinParams* p) {
     return 0;
 }
 
-static int din_smem(int D, size_t* bytes, const void* kernel) {
-    using namespace rk;
-    *bytes = DinSmem::bytes(D);
-    RK_CHECK_ARG(*bytes <= 227 * 1024, "din: %zu bytes of shared memory", *bytes);
-    RK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)*bytes));
-    return 0;
-}
-
 int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float* att_w,
                uint32_t* relu_masks, int32_t* err_flag, rk_stream_t stream_) {
     using namespace rk;
@@ -1960,12 +1567,6 @@ int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float*
     if (int rc = din_pack(args, &p)) return rc;
     RK_CHECK_ARG(concat_all && (att_w || p.T == 0), "din_fwd: NULL output");
     if (p.B == 0) return 0;
-    const int grid = (int)ceil_div(p.B, kSamples);
-    if (p.T > kRows) {
-        RK_CHECK_ARG(args->precision == RK_DIN_FP32, "din_fwd: unknown precision %d", args->precision);
-        return din_launch_long(din_fwd_long_kernel, grid, p.D, stream_, p, concat_all, norm, att_w, relu_masks,
-                               err_flag);
-    }
     if (args->precision == RK_DIN_BF16_TENSOR && p.T > 0) {
         RK_CHECK_ARG(p.D == 16, "din_fwd: the tensor-core activation unit is built for D = 16 (got %d)", p.D);
         const size_t smem_tc = tc::TcFwdSmem::bytes(p.width, p.T, p.cat.F);
@@ -1985,14 +1586,10 @@ int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float*
         RK_LAUNCH_CHECK();
         return 0;
     }
-    // T == 0 (every history empty) runs no activation unit, so both precisions take this kernel
+    // T == 0 (every history empty) runs no activation unit, so both precisions take the fp32 kernel
     RK_CHECK_ARG(args->precision == RK_DIN_FP32 || p.T == 0, "din_fwd: unknown precision %d", args->precision);
-    size_t smem;
-    if (int rc = din_smem(p.D, &smem, (const void*)din_fwd_kernel)) return rc;
-    din_fwd_kernel<<<grid, kDinThreads, smem, (cudaStream_t)stream_>>>(p, concat_all, norm, att_w,
-                                                                       relu_masks, err_flag);
-    RK_LAUNCH_CHECK();
-    return 0;
+    return din_launch(din_fwd_kernel, (int)ceil_div(p.B, kSamples), p.D, stream_, p, concat_all, norm, att_w,
+                      relu_masks, err_flag);
 }
 
 int rk_din_bwd(const rk_din_args_t* args, const float* concat_all, const float* norm,
@@ -2006,11 +1603,6 @@ int rk_din_bwd(const rk_din_args_t* args, const float* concat_all, const float* 
     RK_CHECK_ARG(!g_norm || norm, "din_bwd: g_norm without the saved norms");
     if (p.B == 0) return 0;
     const int grid = (int)ceil_div(p.B, kSamples);
-    if (p.T > kRows) {
-        RK_CHECK_ARG(args->precision == RK_DIN_FP32, "din_bwd: unknown precision %d", args->precision);
-        return din_launch_long(din_bwd_long_kernel, grid, p.D, stream_, p, concat_all, norm, att_w, relu_masks,
-                               g_concat, g_norm, g_row, g_hist, err_flag);
-    }
     if (args->precision == RK_DIN_BF16_TENSOR && p.T > 0) {
         RK_CHECK_ARG(p.D == 16, "din_bwd: the tensor-core activation unit is built for D = 16 (got %d)", p.D);
         const size_t smem_tc = tc::TcBwdSmem::bytes(p.T, p.width);
@@ -2031,12 +1623,9 @@ int rk_din_bwd(const rk_din_args_t* args, const float* concat_all, const float* 
         RK_LAUNCH_CHECK();
         return 0;
     }
-    size_t smem;
-    if (int rc = din_smem(p.D, &smem, (const void*)din_bwd_kernel)) return rc;
-    din_bwd_kernel<<<grid, kDinThreads, smem, (cudaStream_t)stream_>>>(
-        p, concat_all, norm, att_w, relu_masks, g_concat, g_norm, g_row, g_hist, err_flag);
-    RK_LAUNCH_CHECK();
-    return 0;
+    RK_CHECK_ARG(args->precision == RK_DIN_FP32 || p.T == 0, "din_bwd: unknown precision %d", args->precision);
+    return din_launch(din_bwd_kernel, grid, p.D, stream_, p, concat_all, norm, att_w, relu_masks, g_concat, g_norm,
+                      g_row, g_hist, err_flag);
 }
 
 }  // extern "C"

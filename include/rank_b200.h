@@ -208,9 +208,10 @@ typedef struct rk_din_args {
 int rk_din_tile_bytes(void);
 
 int rk_din_mlp_floats(int D);
-/* History width T: any T >= 0 with RK_DIN_FP32.  Up to 128 positions a tile holds whole samples; wider
- * histories are walked by the same CTAs in chunks of at most 128 rows (raw pooling and the softmax's running
- * max / sum carried across chunks in a fixed order: deterministic, no atomics, no host synchronisation).
+/* History width T: any T >= 0 with RK_DIN_FP32.  Its CTAs walk their samples' live positions in tiles of
+ * at most 128 rows: samples of at most 128 positions whole, several to a tile, and a longer sample in chunks
+ * (raw pooling and the softmax's running max / sum carried across chunks in a fixed order: deterministic, no
+ * atomics, no host synchronisation).
  * T = 0 (every history empty) gives an attention output of 0 and needs no att_w / relu_masks / history
  * pointers.  RK_DIN_BF16_TENSOR takes 0 <= T <= 128 and refuses wider histories: use RK_DIN_FP32 there. */
 int rk_din_fwd(const rk_din_args_t* args, float* concat_all, float* norm, float* att_w,

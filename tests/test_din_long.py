@@ -1,12 +1,12 @@
-"""DIN histories wider than one 128-row tile, and batches with no history at all (CPU only).
+"""DIN's fp32 activation unit at every history width, and batches with no history at all (CPU only).
 
 * The C ABI's argument checks for the history width: a negative width and the tensor-core unit above 128
   positions are refused before any CUDA call; width 0 and widths above 128 pass the checks (with B = 0 the
   entry points return before any launch).  Placeholder device addresses, never dereferenced, as in
   test_abi_tiles.py; skipped where a GPU is present.
-* A numpy restatement of the long-history tile planner (plan_long_tile in csrc/din.cu): every live (b, t)
-  row is covered exactly once, in tiles of at most 128 rows, and samples of at most 128 positions are packed
-  whole, exactly as the planner of the 1..128 kernels packs them.
+* A numpy restatement of the fp32 kernels' tile planner (plan_tile in csrc/din.cu): every live (b, t) row is
+  covered exactly once, in tiles of at most 128 rows, and samples of at most 128 positions are packed whole,
+  as many to a tile as fit (so at T <= 128 a tile holds whole samples only).
 """
 import ctypes as C
 
@@ -87,8 +87,8 @@ def test_width_zero_needs_no_history_pointers(call, precision):
 
 
 # ---- the tile planner ---------------------------------------------------------------------------
-def plan_long_tile(lens, s_begin, t_begin):
-    """plan_long_tile (csrc/din.cu): segments [(sample, t0, n)] of the tile and the next cursor."""
+def plan_tile(lens, s_begin, t_begin):
+    """plan_tile (csrc/din.cu): segments [(sample, t0, n)] of the tile and the next cursor."""
     rows, s, t0, segs = 0, s_begin, t_begin, []
     while s < len(lens):
         rem = lens[s] - t0
@@ -109,13 +109,13 @@ def plan_long_tile(lens, s_begin, t_begin):
 def plan_cta(lens):
     tiles, s, t = [], 0, 0
     while s < len(lens):
-        segs, rows, s, t = plan_long_tile(lens, s, t)
+        segs, rows, s, t = plan_tile(lens, s, t)
         tiles.append((segs, rows))
     return tiles
 
 
 def plan_short(lens):
-    """plan_tile of the 1..128 kernels: whole samples while they fit."""
+    """Whole samples while they fit: how samples of at most 128 positions must be packed."""
     tiles, s = [], 0
     while s < len(lens):
         rows, e = 0, s
@@ -128,7 +128,7 @@ def plan_short(lens):
 
 
 def _row_map(segs):
-    """long_row_map: tile row -> (sample, t)."""
+    """row_map: tile row -> (sample, t)."""
     r0 = np.cumsum([0] + [n for _, _, n in segs])
     out = []
     for m in range(r0[-1]):

@@ -1,8 +1,8 @@
 """DIN on histories wider than one 128-row tile (fp32 activation unit), and on batches with no history.
 
-Against the oracle at the 1e-5 fp32 bar with the float64 arbiter of test_gpu_models.py; padding invariance
-between the 1..128 kernels and the long-history kernels; width 0; the index check past position 128; graph
-capture and determinism; the device input path at width 300; and the tensor-core unit's refusal above 128."""
+Against the oracle at the 1e-5 fp32 bar with the float64 arbiter of test_gpu_models.py; invariance of the fp32
+kernels to padding a 128-wide batch past one tile; width 0; the index check past position 128; graph capture
+and determinism; the device input path at width 300; and the tensor-core unit's refusal above 128."""
 import numpy as np
 import pandas as pd
 import pytest
