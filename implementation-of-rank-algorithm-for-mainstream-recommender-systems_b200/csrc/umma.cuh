@@ -1,7 +1,9 @@
-// umma.cuh — tcgen05 / TMEM / mbarrier helpers shared by the tensor-core kernels (din.cu, afm.cu).
-// sm_100a only.  Operands are bf16 tiles in shared memory in the canonical 128-byte-swizzled
-// layouts (8 lines of 128 B form one 1024-byte swizzle atom; the 16-byte chunk index of a line is
-// XORed with line % 8), accumulators are fp32 in TMEM, one elected thread issues the MMAs.
+// umma.cuh — tcgen05 / TMEM / mbarrier helpers shared by the tensor-core kernels (din.cu, afm.cu, linear.cu).
+// sm_100a only.  Operands are bf16 tiles in shared memory in the canonical 128-byte-swizzled layouts (8 lines
+// of 128 B form one 1024-byte swizzle atom; the 16-byte chunk index of a line is XORed with line % 8), or, for
+// the MN-major tf32 operands of linear.cu, the 128B-base-32B layout described at umma_desc_mn_tf32 (4-line,
+// 512-byte atoms; 32-byte granules XORed with line % 4).  Accumulators are fp32 in TMEM, one elected thread
+// issues the MMAs.
 #pragma once
 #include <cuda_bf16.h>
 #include "common.cuh"
@@ -157,6 +159,43 @@ __device__ __forceinline__ uint64_t umma_desc_mn(uint32_t smem_addr, uint32_t mn
     d |= (uint64_t)2 << 61;
     return d;
 }
+// ---- kind::tf32 (fp32 operands rounded to tf32 by the caller, fp32 accumulation) ----
+// MN-major tf32 operands take only the SWIZZLE_128B_BASE32B layout (type 1; CUTLASS's Layout_MN_SW128_32B_Atom):
+// lines of 32 fp32 MN elements (128 bytes), 4 lines form a 512-byte atom in which the 32-byte granule index of
+// a line is XORed with line % 4 (address bits [5,7) ^= [7,9)).  4-line groups are 512 bytes apart (the stride
+// byte offset), so one MMA's K = 8 is two atoms and K advances by +1024 bytes per MMA; blocks of 32 MN
+// elements are `mn_block_bytes` apart (the leading byte offset).
+__device__ __forceinline__ uint64_t umma_desc_mn_tf32(uint32_t smem_addr, uint32_t mn_block_bytes) {
+    uint64_t d = 0;
+    d |= (uint64_t)((smem_addr & 0x3ffff) >> 4);
+    d |= (uint64_t)((mn_block_bytes >> 4) & 0x3fff) << 16;
+    d |= (uint64_t)(512 >> 4) << 32;
+    d |= (uint64_t)1 << 46;
+    d |= (uint64_t)1 << 61;                           // SWIZZLE_128B_BASE32B
+    return d;
+}
+// kind::tf32, A = B = tf32 (format 2 at bits 7 and 10), D = f32, M = 128; OR in kUmmaAMn / kUmmaBMn for MN-major
+__host__ __device__ constexpr uint32_t umma_idesc_tf32(int N) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+}
+__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                          uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+}
+// 3xTF32 split: x = hi + lo exactly, hi = x rounded to tf32 (low 13 mantissa bits zero, ties away from zero).
+// The tensor core reads the top 19 bits of lo, so hi.hi + lo.hi + hi.lo keeps about 22 bits of each operand.
+// A finite |x| within 2^-11 relative of FLT_MAX rounds hi to inf (lo = -inf): far outside any gradient.
+__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
+    uint32_t h;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x));
+    hi = __uint_as_float(h);
+    lo = x - hi;
+}
+
 // asynchronous global -> shared copies (LDGSTS); completion through cp.async.commit_group / wait_group
 __device__ __forceinline__ void cp_async8(const void* dst_smem, const void* src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst_smem)), "l"(src) : "memory");

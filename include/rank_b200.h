@@ -292,7 +292,8 @@ int rk_bn_act_bwd(const float* x, const float* g_z, int64_t B, int units, const 
                   float* g_beta, rk_stream_t stream);
 
 /* Weight and bias gradients of a tower nn.Linear (y = x W^T + b): dW[N, K] = G^T X and db[N] = sum_b G[b, :],
- * fp32 FMA.  Row b of x[B, K] starts at x + b*ldx, of g[B, N] at g + b*ldg (ldx >= K, ldg >= N); db may be
+ * on the tensor core (tcgen05) in 3xTF32 (about 22 bits of every operand, fp32 accumulation), or in fp32 FMA
+ * where the batch is too small to fill half the GPU with tensor-core tiles; db is summed in double.  Row b of x[B, K] starts at x + b*ldx, of g[B, N] at g + b*ldg (ldx >= K, ldg >= N); db may be
  * NULL (no bias).  The batch is split into slabs whose partial sums a second launch adds in a fixed order:
  * partials holds rk_linear_wgrad_scratch_floats(B, K, N) floats (0: may be NULL).  Bit-identical from run to
  * run; no allocation, no synchronisation. */

@@ -5,7 +5,9 @@ For every Linear that run_tower meets in bench.py's workloads (DIN, BST, DCN at 
 times rk_linear_wgrad (csrc/linear.cu) next to what autograd runs (g.t() @ x, then g.sum(0)), each captured in a
 CUDA graph, with L2 warm (the same operands replayed) and flushed (256 MB written between replays, the flush timed
 alone and subtracted).  TFLOP/s count the 2*B*N*K FLOP of dW; the peak is 128 fp32 FMA lanes x 2 per SM at the
-SM clock read in the same run.  --cublas-variants adds the other cuBLAS forms of dW.   python scripts/bench_mm.py
+SM clock read in the same run.  "tf32" is the share of the data-sheet dense TF32 tensor rate of one B200 (1,125
+TFLOP/s) that the three products of rk_linear_wgrad's 3xTF32 scheme (6*B*N*K FLOP) would take at that time.
+--cublas-variants adds the other cuBLAS forms of dW.   python scripts/bench_mm.py
 """
 import argparse
 import os
@@ -23,6 +25,9 @@ SHAPES = {   # workload: (B, [(in, out), ...])
     "dcn": (8192, [(50, 512), (512, 256), (256, 128)]),
     "deepfm": (1024, [(96, 512), (512, 256), (256, 128)]),
 }
+
+
+TF32_DENSE_TFLOPS = 1125.0          # NVIDIA HGX B200 data sheet, one GPU, dense
 
 
 def graph_us(fn, flush=None, n=50):
@@ -96,7 +101,8 @@ def main():
             for key, us in row.items():
                 totals[(work,) + key] = totals.get((work,) + key, 0.0) + us
             print(f"{work:6s} B={B} {k_in:3d}->{n_out:3d}: " + ", ".join(
-                f"{impl} {l2} {us:6.1f} us ({flop / us / 1e6:5.1f} TFLOP/s, {100 * flop / us / 1e6 / peak:4.1f}% peak)"
+                f"{impl} {l2} {us:6.1f} us ({flop / us / 1e6:5.1f} TFLOP/s, {100 * flop / us / 1e6 / peak:4.1f}% peak, "
+                f"tf32 {100 * 3 * flop / us / 1e6 / TF32_DENSE_TFLOPS:4.1f}%)"
                 for (impl, l2), us in row.items()), flush=True)
             if args.cublas_variants:
                 res = {"dW g.t().contiguous()@x": graph_us(lambda: g.t().contiguous() @ x),
