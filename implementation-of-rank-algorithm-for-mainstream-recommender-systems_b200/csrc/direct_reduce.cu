@@ -35,6 +35,7 @@ constexpr int kDirMaxJobs = RK_MAX_FIELDS;
 constexpr int kSeqRun     = 8;                           // runs up to this length: one lane group, in order
 constexpr int kWarpRun    = 128;                         // up to this: one warp; longer: the whole CTA
 constexpr int kDirTarget  = 384;                         // occurrences a CTA should own on average
+constexpr int kDirMaxDim  = 128;                         // widest table row
 
 struct DirectOut {
     const float* g;
@@ -102,7 +103,7 @@ struct RunLists {
 };
 
 // All rows of this CTA's range for one output table.  run_start[d] / run_len[d]: where local row d's
-// occurrences sit in ent[].  red: [kDirWarps][32] floats of scratch.
+// occurrences sit in ent[].  red: [kDirWarps][kDirMaxDim] floats of scratch.
 template <int V>
 __device__ __forceinline__ void reduce_rows(const DirectOut& o, const uint32_t* __restrict__ ent,
                                             const uint32_t* __restrict__ run_start,
@@ -152,7 +153,7 @@ __device__ __forceinline__ void reduce_rows(const DirectOut& o, const uint32_t* 
         }
         if (on && rl == 0) {
 #pragma unroll
-            for (int e = 0; e < V; ++e) red[warp * 32 + cl * V + e] = acc.v[e];
+            for (int e = 0; e < V; ++e) red[warp * kDirMaxDim + cl * V + e] = acc.v[e];
         }
         __syncthreads();
         if (warp == 0 && lane < CL) {
@@ -160,7 +161,7 @@ __device__ __forceinline__ void reduce_rows(const DirectOut& o, const uint32_t* 
             vec_zero(tot);
             for (int ww = 0; ww < kDirWarps; ++ww) {
 #pragma unroll
-                for (int e = 0; e < V; ++e) tot.v[e] += red[ww * 32 + lane * V + e];
+                for (int e = 0; e < V; ++e) tot.v[e] += red[ww * kDirMaxDim + lane * V + e];
             }
             tot.store(o.dw + (int64_t)(row0 + d) * o.dim + lane * V);
         }
@@ -189,7 +190,6 @@ direct_reduce_kernel(const __grid_constant__ DirectParams p, int32_t* err_flag) 
     lists.long_rows  = lists.mid_rows + kDirRows;
     __shared__ int      list_n[3];
     __shared__ uint32_t warp_tot[kDirWarps];
-    __shared__ float    red[kDirWarps * 32];
     lists.n = list_n;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -325,7 +325,9 @@ direct_reduce_kernel(const __grid_constant__ DirectParams p, int32_t* err_flag) 
     }
     __syncthreads();          // also orders the zero stores of step 1 before the sums below
 
-    // 6. the sums
+    // 6. the sums; the long runs' partial rows go where staged[] was (dead from here on)
+    static_assert(kDirWarps * kDirMaxDim <= kDirMaxN, "long-run scratch");
+    float* red = reinterpret_cast<float*>(staged);
     for (int q = 0; q < jb.n_out; ++q) {
         const DirectOut& o = jb.out[q];
         if (o.vec == 4)      reduce_rows<4>(o, ent, run_start, run_len, lists, row0, red);
@@ -358,7 +360,7 @@ int rk_embgrad_direct_reduce(const rk_direct_table_t* tables, int n_tables, int3
     };
     for (int t = 0; t < n_tables; ++t) {
         const rk_direct_table_t& tb = tables[t];
-        RK_CHECK_ARG(tb.dw && tb.rows > 0 && tb.dim > 0 && tb.dim <= 128 && tb.n >= 0, "direct_reduce: table %d rows=%lld dim=%d n=%lld",
+        RK_CHECK_ARG(tb.dw && tb.rows > 0 && tb.dim > 0 && tb.dim <= kDirMaxDim && tb.n >= 0, "direct_reduce: table %d rows=%lld dim=%d n=%lld",
                      t, (long long)tb.rows, tb.dim, (long long)tb.n);
         RK_CHECK_ARG(tb.n <= kDirMaxN, "direct_reduce: table %d has %lld occurrences (max %d: use rk_plan_build + "
                      "rk_embgrad_segment_reduce)", t, (long long)tb.n, kDirMaxN);

@@ -9,6 +9,9 @@
 // (nets[0..N], [B,d] each) for the backward, which recomputes the hidden layer instead of
 // storing it.  Packed per-unit weights (rk_resunit_pack_floats), Hp = roundup(H,8), dp = roundup(d,4):
 //   [W1^T d x Hp][b1 Hp][W2^T Hp x dp][b2 dp][W2 d x Hp][W1 Hp x dp]      (zero padded)
+// Every block must fit the 227 KiB of shared memory a block may have; that, not d, H <= 256 alone,
+// bounds the widths.  The backward takes every (d, H) the forward takes: it stages W1 over W1^T | b1
+// once the hidden layer has been recomputed, and halves its tile height where the block would not fit.
 #include <string.h>
 #include "common.cuh"
 #include "tile_gemm.cuh"
@@ -112,6 +115,11 @@ resunits_fwd_kernel(const __grid_constant__ ResParams p, float* __restrict__ net
     }
 }
 
+// Backward weights: W1^T | b1, later W1 in the same space, then W2.
+__host__ __device__ inline int res_bwd_w1_floats(const ResLayout& L) {
+    return L.d * L.Hp + L.Hp > L.Hp * L.dp ? L.d * L.Hp + L.Hp : L.Hp * L.dp;
+}
+
 __global__ void __launch_bounds__(kResThreads)
 resunits_bwd_kernel(const float* __restrict__ nets, const float* __restrict__ units, int n_units, int H, int d,
                     int rows, int64_t B, const float* __restrict__ g_out, float* __restrict__ g_x0) {
@@ -120,9 +128,9 @@ resunits_bwd_kernel(const float* __restrict__ nets, const float* __restrict__ un
     const int R = rows, ld = R + 4;
     float* W1t = smem_raw;                    // [d][Hp]
     float* b1  = W1t + d * L.Hp;              // [Hp]
-    float* W2  = b1 + L.Hp;                   // [d][Hp]  (as registered: B operand of gz x W2)
-    float* W1  = W2 + d * L.Hp;               // [Hp][dp] (as registered: B operand of gh x W1)
-    float* X   = W1 + L.Hp * L.dp;            // [dp][ld]
+    float* W1  = smem_raw;                    // [Hp][dp] (as registered: B operand of gh x W1), over W1t | b1
+    float* W2  = smem_raw + res_bwd_w1_floats(L);   // [d][Hp]  (as registered: B operand of gz x W2)
+    float* X   = W2 + d * L.Hp;               // [dp][ld]
     float* G   = X + L.dp * ld;               // [dp][ld]
     float* Hs  = G + L.dp * ld;               // [Hp][ld]
     const int tid = threadIdx.x;
@@ -140,7 +148,6 @@ resunits_bwd_kernel(const float* __restrict__ nets, const float* __restrict__ un
         res_copy(W1t, pack + L.w1t, d * L.Hp);
         res_copy(b1, pack + L.b1, L.Hp);
         res_copy(W2, pack + L.w2, d * L.Hp);
-        res_copy(W1, pack + L.w1, L.Hp * L.dp);
         __syncthreads();   // also orders the previous unit's G writes before the reads below
         const float* xin  = nets + (int64_t)u * B * d;
         const float* xout = nets + (int64_t)(u + 1) * B * d;
@@ -158,6 +165,7 @@ resunits_bwd_kernel(const float* __restrict__ nets, const float* __restrict__ un
             store_tile_kmajor<8>(Hs, ld, m0, n0, acc);
         });
         __syncthreads();
+        res_copy(W1, pack + L.w1, L.Hp * L.dp);   // W1^T and b1 are dead from here on
         // gh = (gz x W2) masked by the hidden ReLU, in place over Hs
         tile_gemm<8, kResThreads>(G, ld, W2, L.Hp, d, L.Hp, R, [&](int m0, int n0, float (&acc)[4][8]) {
 #pragma unroll
@@ -188,7 +196,17 @@ resunits_bwd_kernel(const float* __restrict__ nets, const float* __restrict__ un
     }
 }
 
+constexpr size_t kResSmemMax = 227 * 1024;   // dynamic shared memory a block may have
+
 static int res_rows(int H) { return H > 128 ? 32 : 64; }
+
+static size_t res_fwd_smem(const ResLayout& L, int rows) {
+    return sizeof(float) * ((size_t)L.w2 + (size_t)(L.dp + L.Hp) * (rows + 4));
+}
+
+static size_t res_bwd_smem(const ResLayout& L, int rows) {
+    return sizeof(float) * ((size_t)res_bwd_w1_floats(L) + (size_t)L.d * L.Hp + (size_t)(2 * L.dp + L.Hp) * (rows + 4));
+}
 
 }  // namespace rk
 
@@ -212,14 +230,15 @@ int rk_resunits_fwd(const rk_field_t* fields, int F, const float* dense, int n_d
     for (int f = 0; f < F; ++f) covered += fields[f].dim;
     RK_CHECK_ARG(covered == d, "resunits: the fields do not tile the %d-wide row", d);
     RK_CHECK_ARG(d >= 1 && d <= 256 && H >= 1 && H <= 256 && n_units >= 0,
-                 "resunits: d=%d H=%d units=%d (supported: d,H <= 256)", d, H, n_units);
+                 "resunits: d=%d H=%d units=%d (d and H must lie in [1, 256], units >= 0)", d, H, n_units);
     RK_CHECK_ARG(nets && (n_units == 0 || units), "resunits: NULL pointer");
     if (B == 0) return 0;
     p.dense = dense; p.units = units; p.n_dense = n_dense; p.d = d; p.H = H; p.n_units = n_units;
     p.rows = res_rows(H); p.B = B;
     const ResLayout L(d, H);
-    const size_t smem = sizeof(float) * ((size_t)L.w2 + (size_t)(L.dp + L.Hp) * (p.rows + 4));
-    RK_CHECK_ARG(smem <= 227 * 1024, "resunits_fwd: %zu bytes of shared memory", smem);
+    const size_t smem = res_fwd_smem(L, p.rows);
+    RK_CHECK_ARG(smem <= kResSmemMax, "resunits_fwd: d=%d H=%d needs %zu bytes of shared memory, a block may have %zu",
+                 d, H, smem, kResSmemMax);
     RK_CUDA(cudaFuncSetAttribute(resunits_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     resunits_fwd_kernel<<<(int)ceil_div(B, p.rows), kResThreads, smem, (cudaStream_t)stream_>>>(p, nets, err_flag);
     RK_LAUNCH_CHECK();
@@ -230,13 +249,15 @@ int rk_resunits_bwd(const float* nets, const float* units, int n_units, int H, i
                     const float* g_out, float* g_x0, rk_stream_t stream_) {
     using namespace rk;
     RK_CHECK_ARG(nets && g_out && g_x0 && (n_units == 0 || units), "resunits_bwd: NULL pointer");
-    RK_CHECK_ARG(d >= 1 && d <= 256 && H >= 1 && H <= 256 && n_units >= 0, "resunits_bwd: d=%d H=%d", d, H);
+    RK_CHECK_ARG(d >= 1 && d <= 256 && H >= 1 && H <= 256 && n_units >= 0,
+                 "resunits_bwd: d=%d H=%d units=%d (d and H must lie in [1, 256], units >= 0)", d, H, n_units);
     if (B == 0) return 0;
-    const int rows = res_rows(H);
     const ResLayout L(d, H);
-    const size_t smem = sizeof(float) * ((size_t)2 * d * L.Hp + L.Hp + (size_t)L.Hp * L.dp +
-                                         (size_t)(2 * L.dp + L.Hp) * (rows + 4));
-    RK_CHECK_ARG(smem <= 227 * 1024, "resunits_bwd: %zu bytes of shared memory", smem);
+    int rows = res_rows(H);
+    while (rows > 4 && res_bwd_smem(L, rows) > kResSmemMax) rows >>= 1;
+    const size_t smem = res_bwd_smem(L, rows);
+    RK_CHECK_ARG(smem <= kResSmemMax, "resunits_bwd: d=%d H=%d needs %zu bytes of shared memory, a block may have %zu",
+                 d, H, smem, kResSmemMax);
     RK_CUDA(cudaFuncSetAttribute(resunits_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     resunits_bwd_kernel<<<(int)ceil_div(B, rows), kResThreads, smem, (cudaStream_t)stream_>>>(
         nets, units, n_units, H, d, rows, B, g_out, g_x0);

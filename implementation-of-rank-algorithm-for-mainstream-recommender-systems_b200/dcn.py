@@ -18,7 +18,7 @@ import torch.nn as nn
 
 from . import _lib
 from .ephemeral import EphemeralBuffer
-from .sparse import GradSource, OccurrencePlan, field_array
+from .sparse import GradSource, OccurrencePlan, check_table_gradients, field_array
 from .tower import run_tower
 from .vocab import table_heights
 
@@ -64,6 +64,8 @@ class _CrossNet(torch.autograd.Function):
         for i in idx:
             if i.shape != (B,):
                 raise ValueError("every category column must be [batch]")
+        if any(ctx.needs_input_grad[5 + F:]):
+            check_table_gradients([(int(t.shape[1]), o, d) for o, t in zip(offsets, tables)], "CrossNet")
         dev = dense.device
         concat_all = torch.empty(B, d, dtype=torch.float32, device=dev)
         cross_vec = torch.empty(B, d, dtype=torch.float32, device=dev)

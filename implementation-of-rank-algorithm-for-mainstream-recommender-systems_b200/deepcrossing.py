@@ -20,7 +20,7 @@ import torch.nn.functional as Fn
 from . import _lib
 from .dcn import NUM_DENSE, SIDE_COLUMNS, SIDE_TABLES
 from .ephemeral import EphemeralBuffer
-from .sparse import GradSource, OccurrencePlan, field_array
+from .sparse import GradSource, OccurrencePlan, check_table_gradients, field_array
 from .vocab import table_heights
 
 
@@ -57,6 +57,8 @@ class _ResidualStack(torch.autograd.Function):
         dense = _lib.require_cuda(dense, "dense", torch.float32)
         B, n_dense = int(dense.shape[0]), int(dense.shape[1])
         d = max([n_dense] + [o + int(t.shape[1]) for o, t in zip(offsets, tables)])
+        if any(ctx.needs_input_grad[6 + F:]):
+            check_table_gradients([(int(t.shape[1]), o, d) for o, t in zip(offsets, tables)], "residual units")
         dev = dense.device
         if n_units:
             units = _lib.require_cuda(units, "residual weights", torch.float32)

@@ -15,7 +15,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .sparse import GradSource, OccurrencePlan, field_array
+from .sparse import GradSource, OccurrencePlan, check_table_gradients, field_array
 from .tower import run_tower
 from .vocab import table_heights
 
@@ -35,6 +35,9 @@ class _FMInteraction(torch.autograd.Function):
             if w.shape != (second[f].shape[0], 1):
                 raise ValueError(f"first-order table {f} must be [{second[f].shape[0]}, 1]")
         B, D = int(idx[0].shape[0]), int(second[0].shape[1])
+        if any(ctx.needs_input_grad):
+            # the backward reduces the F second-order and the F first-order gradients together
+            check_table_gradients([(D, f * D, F * D) for f in range(F)] + [(1, 0, 1)] * F, "FM part")
         dev = second[0].device
         deep_input = torch.empty(B, F * D, dtype=torch.float32, device=dev)
         fm_first = torch.empty(B, 1, dtype=torch.float32, device=dev)

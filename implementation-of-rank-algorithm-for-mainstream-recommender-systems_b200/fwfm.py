@@ -16,7 +16,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .sparse import GradSource, OccurrencePlan, field_array
+from .sparse import GradSource, OccurrencePlan, check_table_gradients, field_array
 
 FWFM_COLUMNS = ("userid", "feedid", "device", "authorid", "bgm_song_id", "bgm_singer_id")
 
@@ -40,6 +40,9 @@ class _FwFMInteraction(torch.autograd.Function):
         if field_weight.numel() != P or bias.numel() != 1:
             raise ValueError(f"field_weight must have {P} entries and bias 1")
         B, D = int(idx[0].shape[0]), int(second[0].shape[1])
+        if any(ctx.needs_input_grad):
+            # the backward reduces the F embedding and the F linear-table gradients together
+            check_table_gradients([(D, f * D, F * D) for f in range(F)] + [(1, 0, 1)] * F, "FwFM")
         dev = second[0].device
         emb = torch.empty(B, F * D, dtype=torch.float32, device=dev)
         y = torch.empty(B, dtype=torch.float32, device=dev)

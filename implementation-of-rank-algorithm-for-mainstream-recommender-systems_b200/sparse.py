@@ -76,6 +76,26 @@ class GradSource:
     param: object = None  # the table tensor itself (where a touched-rows gradient is attached)
 
 
+def check_table_gradients(tables, what):
+    """Refuse, before the forward launches anything, a layout whose table gradients the backward's
+    reductions (rk_embgrad_direct_reduce, rk_embgrad_segment_reduce) would refuse.  `tables` lists the
+    (dim, offset, ld) of every GradSource the backward will hand to OccurrencePlan.reduce_to_dense.
+    * at most RK_MAX_TABLES gradient tables in one reduction;
+    * a reduction lane carries 4, 2 or 1 floats, the widest that divides the row's dim, its offset and
+      the row pitch ld, and a row has at most 32 lanes: dim <= 32 * that width."""
+    if len(tables) > _lib.RK_MAX_TABLES:
+        raise _lib.RankB200Error(f"{what}: the backward reduces {len(tables)} gradient tables "
+                                 f"(at most RK_MAX_TABLES={_lib.RK_MAX_TABLES})")
+    for t, (dim, offset, ld) in enumerate(tables):
+        vec = 4
+        while vec > 1 and (dim % vec or offset % vec or ld % vec):
+            vec //= 2
+        if dim > 32 * vec:
+            raise _lib.RankB200Error(
+                f"{what}: table {t} is {dim} floats wide at column {offset} of a {ld}-float row; its gradient "
+                f"reduction moves {vec} float(s) per lane, 32 lanes, so at most {32 * vec} columns")
+
+
 # ---- opt-in sparse gradients of the replicated tables (SURVEY 8(f) item 3) ---------------------
 # "dense"  : every table receives a dense [V, D] .grad, as the reference's nn.Embedding(sparse=False)
 #            does (DeepFM/deepfm.py:90-98) and dense optim.Adam needs (:226) — the default.

@@ -382,7 +382,9 @@ int rk_plan_compact_fields(const uint32_t* sorted_keys, const int64_t* n, const 
  *   [W1^T d x Hp][b1 Hp][W2^T Hp x dp][b2 dp][W2 d x Hp][W1 Hp x dp], Hp = roundup(H,8),
  *   dp = roundup(d,4), zero padded (W1 [H,d], W2 [d,H] as nn.Linear stores them).
  * nets[(n_units+1), B, d]: nets[0] = the concat row, nets[i+1] = output of unit i (the last one
- * is the result; all are kept for the backward).  bwd: g_x0[B,d] = d(loss)/d(nets[0]). */
+ * is the result; all are kept for the backward).  bwd: g_x0[B,d] = d(loss)/d(nets[0]).
+ * 1 <= d, H <= 256, and the forward's block must fit the 227 KiB of shared memory a block may have
+ * (e.g. d <= 151 at H = 128, d <= 88 at H = 256); the backward takes every (d, H) the forward takes. */
 int rk_resunit_pack_floats(int d, int H);
 int rk_resunits_fwd(const rk_field_t* fields, int F, const float* dense, int n_dense,
                     const float* units, int n_units, int H, int64_t B, float* nets,

@@ -76,6 +76,23 @@ def test_segment_reduce_matches_sequential_sum(n, rows, dim, direct):
 
 
 @pytest.mark.parametrize("direct", [True, False], ids=["direct", "sorted"])
+@pytest.mark.parametrize("n,rows,dim", [(8192, 23, 128), (5000, 3, 64), (3000, 40, 36), (8192, 2, 100),
+                                         (4000, 5, 50)])
+def test_reduce_wide_rows_hit_hundreds_of_times(n, rows, dim, direct):
+    """Rows wider than 32 floats (2 or 4 per lane) whose runs are longer than a warp's share, so that every
+    warp of the CTA sums a slice of the same row (a DeepFM embedding of 64 or 128 and its `device` field)."""
+    gen = torch.Generator().manual_seed(n + dim)
+    idx = torch.randint(0, rows, (n,), generator=gen, dtype=torch.int64)
+    off = 4 if dim % 4 == 0 else 2
+    ld = dim + off
+    g = torch.randn(n, ld, generator=gen)
+    plan = OccurrencePlan([idx.to(DEV)], [rows], direct=direct)
+    (dw,) = plan.reduce_to_dense([GradSource(g.to(DEV), off, ld, dim, rows, 0)])
+    want = X.dense_embedding_grad(idx.numpy(), g[:, off:off + dim].numpy(), rows)
+    assert np.allclose(dw.cpu().numpy(), want, rtol=1e-5, atol=1e-5 * np.abs(want).max())
+
+
+@pytest.mark.parametrize("direct", [True, False], ids=["direct", "sorted"])
 def test_segment_reduce_is_deterministic_and_shares_a_plan(direct):
     gen = torch.Generator().manual_seed(5)
     idx = [torch.randint(0, r, (4096,), generator=gen, dtype=torch.int64).to(DEV) for r in (3, 1000)]
